@@ -283,6 +283,15 @@ def pack_segments(segs):
     return blob, off
 
 
+def dump_outputs(out_dir, recs, roff):
+    """What the last timed step returned to its caller (sd_fetch_staged): every record field and the per-segment record
+    offsets, as float64 (exact for these int32 / int64 values), so that two builds can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name in recs.dtype.names:
+        np.save(os.path.join(out_dir, "records_%s.npy" % name), recs[name].astype(np.float64))
+    np.save(os.path.join(out_dir, "record_offsets.npy"), roff.astype(np.float64))
+
+
 _OUT = None
 
 
@@ -301,7 +310,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the rescoring / process / replica extras")
     ap.add_argument("--geom", default=None, help="override launch geometry C,T,NS (exploration)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the records of the last timed step as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the outputs of --impl ours")
     # stdout carries the one JSON line and nothing else: native libraries that write to file descriptor 1 (NCCL prints
     # its version banner there when NCCL_DEBUG is set) are sent to stderr, the line goes to the saved descriptor
     global _OUT
@@ -336,6 +351,8 @@ def main():
         flushes = [torch.empty(256 << 20, dtype=torch.uint8, device="cuda:%d" % d) for d in range(ws)]
         dev_ms, wall, clocks, st = timed_resident(dec, packed, args, ws, flushes, local)
         recs, roff = dec.fetch_staged()
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, recs, roff)
         e2e_s, st2, r2, o2, e2e_py_s = timed_e2e(dec, packed, args, ws)
         same = bool(len(r2) == len(recs) and (r2 == recs).all() and (o2 == roff).all())
         value = cells_hl * args.steps / (dev_ms * 1e-3) / 1e9

@@ -20,6 +20,23 @@ def load_cases():
         return json.load(f)["cases"]
 
 
+def write_config2(directory):
+    """BASELINE config 2 in full (one 2 Mb array, 80-column FASTA) and its 12 monomers -> (reads path, monomers path)."""
+    from stringdecomposer_b200 import synth
+    rn, reads, mn, mons = synth.config2()
+    rp, mp = os.path.join(str(directory), "reads.fa"), os.path.join(str(directory), "monomers.fa")
+    synth.write_fasta(rp, rn, reads, width=80)
+    synth.write_fasta(mp, mn, mons)
+    return rp, mp
+
+
+def config5_sample():
+    """BASELINE config 5's 1,000 monomers against the first 3,700 bp of one of its arrays -> (names, reads, names, monomers)."""
+    from stringdecomposer_b200 import synth
+    rn, reads, mn, mons = synth.config5(n_monomers=1000, total=40_000)
+    return rn[:1], [reads[0][:3700]], mn, mons
+
+
 def run_case(binary, case, env=None):
     """-> (status, stdout, stderr) of `binary` on a golden case, temp paths stripped from stderr."""
     e = dict(os.environ)

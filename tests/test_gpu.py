@@ -1,8 +1,11 @@
 """GPU parity tests (run on the B200 box with -m gpu).  Everything goes through the C ABI (libsd_b200.so) or the
 drop-in dp binary; the oracle is only the checker."""
 import hashlib
+import json
 import os
 import subprocess
+import sys
+import textwrap
 
 import numpy as np
 import pytest
@@ -20,12 +23,20 @@ def as_tuples(recs):
 
 
 def test_native_library_is_the_one_running():
-    d = Decomposer(["ACGTACGTAC"], devices=[0])
-    recs, off = d.decompose(["ACGTACGTACGGTACGTAC"])
-    st = d.stats()
-    assert st["launches"] >= 2 and st["n_devices"] == 1 and st["cells"] == 19 * 20
-    maps = open("/proc/self/maps").read()
-    assert "libsd_b200.so" in maps and "libsd_emu.so" not in maps
+    # in a fresh interpreter: the CPU tests of a whole-suite run load the host emulator into this process
+    code = textwrap.dedent("""
+        import sys
+        sys.path.insert(0, %r)
+        from stringdecomposer_b200 import Decomposer
+        d = Decomposer(["ACGTACGTAC"], devices=[0])
+        recs, off = d.decompose(["ACGTACGTACGGTACGTAC"])
+        st = d.stats()
+        assert st["launches"] >= 2 and st["n_devices"] == 1 and st["cells"] == 19 * 20
+        maps = open("/proc/self/maps").read()
+        assert "libsd_b200.so" in maps and "libsd_emu.so" not in maps
+    """) % cases.ROOT
+    p = subprocess.run([sys.executable, "-c", code], stdout=subprocess.PIPE, stderr=subprocess.PIPE)
+    assert p.returncode == 0, p.stderr.decode()[-2000:]
 
 
 @pytest.mark.parametrize("scoring,fixture", [(None, "config1_raw_default.tsv"), ((-2, -2, -3, 1), "config1_raw_s-2-2-3+1.tsv")])
@@ -181,19 +192,20 @@ def test_config2_full_size_properties_and_sampled_parity():
     d.close()
 
 
-@pytest.mark.skipif(not os.path.exists(cases.DP_REF), reason="the compiled reference binary (oracle/_ref/dp) is not here")
 def test_config2_full_output_identical_to_the_reference_binary(tmp_path):
-    # BASELINE config 2 in full through both binaries: the unmodified reference needs ~4 s on 16 cores for it
-    rn, reads, mn, mons = synth.config2()
-    rp, mp = str(tmp_path / "reads.fa"), str(tmp_path / "monomers.fa")
-    synth.write_fasta(rp, rn, reads, width=80)
-    synth.write_fasta(mp, mn, mons)
-    tail = [str(os.cpu_count() or 1), "5000", "500"]
-    ours = subprocess.run([cases.DP_CUDA, rp, mp] + tail, stdout=subprocess.PIPE, stderr=subprocess.PIPE)
-    ref = subprocess.run([cases.DP_REF, rp, mp] + tail, stdout=subprocess.PIPE, stderr=subprocess.PIPE)
-    assert ours.returncode == 0 and ref.returncode == 0
-    assert ours.stdout == ref.stdout and ours.stdout.count(b"\n") > 11000
-    assert [ln for ln in ours.stderr.splitlines() if not ln.startswith(b"[sd_b200]")] == ref.stderr.splitlines()
+    # BASELINE config 2 in full through the dp binary, against what the unmodified reference prints for it
+    # (tests/golden/make_golden_full_runs.py: its size and MD5, a sample of its lines, its stderr)
+    with open(os.path.join(cases.GOLDEN, "config2_raw_digest.json")) as f:
+        ref = json.load(f)
+    rp, mp = cases.write_config2(tmp_path)
+    ours = subprocess.run([cases.DP_CUDA, rp, mp, str(os.cpu_count() or 1), "5000", "500"], stdout=subprocess.PIPE, stderr=subprocess.PIPE)
+    assert ours.returncode == 0
+    lines = ours.stdout.decode().splitlines(True)
+    for i, want in ref["sample"]:
+        assert i < len(lines) and lines[i] == want, "raw TSV line %d differs from the reference" % i
+    assert len(ours.stdout) == ref["bytes"] and len(lines) == ref["lines"] > 11000
+    assert hashlib.md5(ours.stdout).hexdigest() == ref["md5"]
+    assert [ln for ln in ours.stderr.decode().splitlines() if not ln.startswith("[sd_b200]")] == ref["stderr"]
 
 
 def test_config4_custom_scoring_sample():
@@ -331,11 +343,10 @@ def test_config5_full_monomer_set_against_the_reference_binary():
     # BASELINE config 5 at its defining scale: 1,000 monomers -> 2,000 DP rows, sum(L) = 342 kb, which the planner spreads
     # over 32 partner CTAs per segment (group sweep).  The reference needs n * sum(L) * 8 B per segment in flight
     # (5.5 GB for a 2,000-column segment), so parity is checked on two 2,000-column segments plus a short tail, against
-    # the unmodified reference binary where it travelled with the snapshot (else against the oracle's C restatement).
-    rn, reads, mn, mons = synth.config5(n_monomers=1000, total=40_000)
-    read = reads[0][:3700]
-    binary = cases.DP_REF if os.path.exists(cases.DP_REF) else None
-    want = sd_oracle.decompose_reads(rn[:1], [read], mn, mons, part_size=1700, overlap=300, binary=binary, threads=2)
+    # the raw TSV the unmodified reference binary prints for them (tests/golden/make_golden_full_runs.py).
+    rn, (read,), mn, mons = cases.config5_sample()
+    with open(os.path.join(cases.GOLDEN, "config5_1000_monomers_raw.tsv"), newline="") as f:
+        want = f.read()
     d = Decomposer(mons, devices=[0])
     segs, _ = segment_reads([read], 1700, 300)
     assert [len(x) for x in segs] == [2000, 2000, 300]
