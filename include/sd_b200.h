@@ -23,7 +23,8 @@ enum {
     SD_ERR_ARG = 1,          /* bad argument (NULL, negative size, symbol outside ACGTN, ...) */
     SD_ERR_NO_DEVICE = 2,    /* no usable CUDA device / CUDA runtime error at start-up */
     SD_ERR_UNSUPPORTED = 3,  /* outside the supported domain (monomer set too large for this build, scores reaching
-                                the reference's INF sentinel, a sequence too long for sd_identity) */
+                                the reference's INF sentinel, a segment whose DP needs more device memory than the
+                                device has, a sequence too long for sd_identity) */
     SD_ERR_CUDA = 4,         /* CUDA failure while running */
     SD_ERR_INTERNAL = 5,
     SD_ERR_INPUT = 255       /* illegal FASTA symbol: the reference exits with status 255 (main.cpp:333-336) */
@@ -45,7 +46,9 @@ typedef struct {
     int32_t n_devices;
     int32_t packed;                     /* 1: s16x2 sweep, 0: s32 sweep (last call) */
     int32_t C, T, NS, NT;               /* launch geometry of the last call */
-    int32_t NG, lat, scanw, pad_;       /* CTAs per segment; 1 = deferred-jump sweep; carry window of the scan */
+    int32_t NG, lat, scanw;             /* CTAs per segment; 1 = deferred-jump sweep; carry window of the scan */
+    int32_t stream;                     /* 1: the sweep read the segment symbols from global memory as it went (segments
+                                           too long for shared memory); 0: they were staged in shared memory */
     int64_t sweep_store_bytes;          /* bytes the sweep writes per pass over the last batch: 2-bit codes (incl. slot
                                            padding) + 8 B per column, summed over devices -- computed from the layout */
     int32_t dev_segments[8];            /* segments each device got in the last batch (AlignReadsSet's gather,
@@ -63,7 +66,14 @@ int sd_create(const char *monomers, const int64_t *offsets, int32_t n_monomers,
 /* Replaces the per-segment calls of AlignPartClassicDP (main.cpp:151-270) that AlignReadsSet issues under OpenMP
  * (main.cpp:87-102).  segments: ACGTN text of all segments back to back, segment s = [offsets[s], offsets[s+1]).
  * On success *records holds the alignments of all segments in segment order, each segment's in read order,
- * and (*rec_offsets)[s .. s+1] delimits segment s (n_segments+1 entries).  Release both with sd_free(). */
+ * and (*rec_offsets)[s .. s+1] delimits segment s (n_segments+1 entries).  Release both with sd_free().
+ * Segment length is limited only by the score domain and by device memory, not by shared memory: segments too long to
+ * be staged in shared memory are swept with their symbols read from device memory (sd_stats.stream).  A segment whose
+ * scores can reach the reference's INF sentinel -- length * max(|ins|, |mismatch|) + 2 * longest monomer * |del| +
+ * 2 * |mismatch| + |match| must stay below 999,000, about 998 kb with the default scores -- returns
+ * SD_ERR_UNSUPPORTED, and so does a segment whose backpointers (0.25 B per cell of every monomer row, with slot
+ * padding) exceed the memory that was free on its device when the handle was created; sd_last_error() then gives the
+ * segment length and the bytes needed and available. */
 int sd_decompose(sd_handle *h, const char *segments, const int64_t *offsets, int64_t n_segments,
                  sd_record **records, int64_t **rec_offsets);
 
@@ -84,7 +94,9 @@ int64_t sd_postprocess(const sd_record *in, int64_t n, sd_record *out);
 /* Replaces main() of the `dp` binary (main.cpp:374-402) after argument parsing: load_fasta of both files
  * (main.cpp:314-346), reverse complements, segmentation, DP, overlap resolution, SaveBatch (main.cpp:272-285).
  * The raw TSV goes to out_fd, the reference's diagnostics to err_fd.  Returns the process exit status the
- * reference would produce (0, or 255 for an illegal symbol) or an SD_ERR_* code. */
+ * reference would produce (0, or 255 for an illegal symbol) or an SD_ERR_* code.  part_size may be as large as the
+ * longest read (one segment per read); the segment-length limits of sd_decompose apply, and both return
+ * SD_ERR_UNSUPPORTED (3) with an "ERROR: ..." line on err_fd and no output. */
 int sd_run_files(const char *reads_path, const char *monomers_path, int32_t threads, int32_t part_size,
                  int32_t overlap, int32_t ins, int32_t del, int32_t mismatch, int32_t match, int32_t ed_thr,
                  int out_fd, int err_fd);

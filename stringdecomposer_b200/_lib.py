@@ -20,7 +20,7 @@ class _Stats(C.Structure):
                 ("h2d_bytes", C.c_int64), ("d2h_bytes", C.c_int64), ("cells", C.c_int64), ("segments", C.c_int64),
                 ("columns", C.c_int64), ("launches", C.c_int64), ("n_devices", C.c_int32), ("packed", C.c_int32),
                 ("C", C.c_int32), ("T", C.c_int32), ("NS", C.c_int32), ("NT", C.c_int32),
-                ("NG", C.c_int32), ("lat", C.c_int32), ("scanw", C.c_int32), ("pad_", C.c_int32),
+                ("NG", C.c_int32), ("lat", C.c_int32), ("scanw", C.c_int32), ("stream", C.c_int32),
                 ("sweep_store_bytes", C.c_int64), ("dev_segments", C.c_int32 * 8)]
 
 
@@ -252,7 +252,7 @@ class Decomposer:
     def stats(self):
         s = _Stats()
         self._lib.sd_get_stats(self._h, C.byref(s))
-        d = {k: getattr(s, k) for k, _ in _Stats._fields_ if k != "pad_"}
+        d = {k: getattr(s, k) for k, _ in _Stats._fields_}
         d["dev_segments"] = [int(x) for x in d["dev_segments"]][:max(1, d["n_devices"])]
         return d
 

@@ -5,6 +5,9 @@ and the identity rescoring through ``sd_identity``.  Needs neither Biopython nor
 
     python -m stringdecomposer_b200 reads.fa monomers.fa -o out_dir [--second-best] [-s ins,del,mm,match] ...
 
+``--whole-reads`` sets the segment size (``-b``) to the longest read of the file, so that every read is decomposed as
+one segment, with no segment seams for the overlap resolution to patch.
+
 writes ``<out-dir>/<out-file>_raw.tsv``, ``<out-file>.tsv``, ``<out-file>_alt.tsv`` and ``stringdecomposer.log``.
 
 Scoring: the reference's main.py always passes ten arguments to `dp`, which parses the scores only when it gets nine
@@ -78,6 +81,8 @@ def main(argv=None, flavour="cuda"):
     parser.add_argument("--second-best", dest="second_best", help="generate second best monomer and homopolymer scores", action="store_true")
     parser.add_argument("--ed_thr", help="align only monomers with edit distance less then ed_thr for each segment (by default align all monomers)",
                         default=-1, type=int, required=False)
+    parser.add_argument("--whole-reads", dest="whole_reads", action="store_true",
+                        help="decompose every read as one segment: the segment size becomes the longest read (overrides -b)")
     parser.add_argument("-v", "--overlap", help="size of the segment overlap (by default 500)", type=str, default="500", required=False)
     parser.add_argument("--device", help="CUDA device of the identity stage (by default 0; the DP obeys SD_DEVICES)", type=int, default=0)
     args = parser.parse_args(argv)
@@ -88,12 +93,19 @@ def main(argv=None, flavour="cuda"):
 
     raw_fn = os.path.join(args.out_dir, args.out_file + "_raw.tsv")
     t0 = time.time()
-    run(args.sequences, args.monomers, args.threads, args.scoring, args.batch_size, raw_fn, args.ed_thr, args.overlap,
+    reads = None
+    batch_size = args.batch_size
+    if args.whole_reads:
+        reads = load_fasta(args.sequences, "map")
+        batch_size = str(max([len(s) for s in reads.values()] + [1]))
+        logger.info("--whole-reads: segment size %s (the longest read), every read is one segment" % batch_size)
+    run(args.sequences, args.monomers, args.threads, args.scoring, batch_size, raw_fn, args.ed_thr, args.overlap,
               logger, flavour=flavour)
     t1 = time.time()
     logger.info("Saved raw decomposition to " + raw_fn)
 
-    reads = load_fasta(args.sequences, "map")
+    if reads is None:
+        reads = load_fasta(args.sequences, "map")
     monomers = add_rc_monomers(load_fasta(args.monomers))
     logger.info("Transforming raw alignments...")
     out_fn = os.path.join(args.out_dir, args.out_file + ".tsv")

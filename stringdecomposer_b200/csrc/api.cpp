@@ -278,7 +278,7 @@ int sd_get_stats(sd_handle *h, sd_stats *o)
     o->h2d_bytes = s.h2d_bytes; o->d2h_bytes = s.d2h_bytes; o->cells = s.cells; o->segments = s.segments;
     o->columns = s.columns; o->launches = s.launches; o->n_devices = h->n_devices;
     o->packed = s.g.packed; o->C = s.g.C; o->T = s.g.T; o->NS = s.g.NS; o->NT = s.g.NT;
-    o->NG = s.g.NG; o->lat = s.g.lat; o->scanw = s.g.scanw;
+    o->NG = s.g.NG; o->lat = s.g.lat; o->scanw = s.g.scanw; o->stream = s.g.stream;
     o->sweep_store_bytes = s.sweep_store_bytes;
     for (int d = 0; d < 8; ++d) o->dev_segments[d] = s.dev_segments[d];
     return SD_OK;

@@ -100,6 +100,9 @@ public:
     virtual void configure(const Plan &p, const MonomerSet &ms) = 0;
     virtual int64_t wave_bytes(const Batch &b, int seg_begin, int seg_end) const = 0;   // device bytes stage() would need
     virtual int64_t wave_budget() const = 0;                                            // bytes one wave may use
+    // device memory a wave can never exceed: the CUDA backend reports what was free when it was created (never the
+    // SD_WAVE_BYTES override); the host emulator keeps the fixed 1 GiB its wave budget was written for
+    virtual int64_t device_bytes() const { return (int64_t)1 << 30; }
     // --ed_thr pre-filter (FilterMonomersForRead, main.cpp:135-149): -1 = off.  Applied by stage() to every segment.
     virtual void set_filter(int ed_thr) { ed_thr_ = ed_thr; }
     virtual void stage(const Batch &b, int seg_begin, int seg_end) = 0;

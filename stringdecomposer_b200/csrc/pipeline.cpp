@@ -322,6 +322,25 @@ void Engine::split(const Batch &b, std::vector<int> &bounds) const
     }
 }
 
+// The wave loop below forms a wave of at least NS segments (one CTA) even when that exceeds the soft wave budget.  Such a
+// minimum wave that exceeds the memory the device had free is refused up front, before anything is allocated, instead
+// of failing in the middle of a run.  Every minimum wave is one of the NS-aligned blocks of a device's range.
+static void check_device_fit(const Backend &dev, const Batch &b, int s0, int s1, int NS)
+{
+    const int64_t cap = dev.device_bytes();
+    for (int s = s0; s < s1; s += NS) {
+        const int e = std::min(s1, s + NS);
+        const int64_t need = dev.wave_bytes(b, s, e);
+        if (need <= cap) continue;
+        int longest = 0;
+        for (int q = s; q < e; ++q) longest = std::max(longest, b.len(q));
+        char msg[256];
+        snprintf(msg, sizeof msg, "segment of %d bp needs %lld bytes of device memory for its sweep; %lld bytes are available "
+                 "(segment the reads with a smaller -b)", longest, (long long)need, (long long)cap);
+        throw PlanError{msg};
+    }
+}
+
 void Engine::decompose(const Batch &b, BatchResult &out)
 {
     out.recs.clear(); out.rec_off.assign(1, 0);
@@ -331,6 +350,7 @@ void Engine::decompose(const Batch &b, BatchResult &out)
     std::vector<int> bounds; split(b, bounds);
     note_split(b, bounds);
     const int nd = ndev();
+    for (int d = 0; d < nd; ++d) check_device_fit(*devs_[d], b, bounds[d], bounds[d + 1], plan_.g.NS);
     std::vector<BatchResult> part(nd);
     std::vector<std::string> errs(nd);
     auto work = [&](int d) {

@@ -186,32 +186,37 @@ Plan make_plan(const MonomerSet &ms, const Scoring &sc, int max_seg_len, int64_t
     int bestC = 0, bestT = 0, bestNS = 0, bestNT = 0; double best = 1e300;
     int fC = 0, fT = 0, fNS = 0;
     if (const char *e = getenv("SD_GEOM")) sscanf(e, "%d,%d,%d", &fC, &fT, &fNS);
+    // Symbols of the segments: staged in shared memory (NS * (max_seg_len + 64) bytes) wherever that fits, streamed from
+    // global memory (no length term) where it does not.  SD_STREAM_SYMBOLS=1 (tests) streams on every shape.
+    const bool force_stream = getenv("SD_STREAM_SYMBOLS") && atoi(getenv("SD_STREAM_SYMBOLS")) > 0;
+    int stream = force_stream ? 1 : 0;
     // lanes with more than 24 cells run into register-limited occupancy and long dependent chains (measured);
     // they are only considered for rows that need them
     const bool need_big = ms.Lmax > 24 * 32;
-    for (int C : kC) for (int T : kT) {
-        if (fC && (C != fC || T != fT)) continue;
-        if (C * T < ms.Lmax) continue;
-        if (!fC && C > 24 && !need_big) continue;
-        int ls = nslots * T;                        // lanes per segment
-        if (ls > 1024) continue;
-        const int qpc = ((C + 3) / 4) | 1;
-        size_t prof_bytes = (size_t)5 * qpc * ls * 16;
-        for (int NS = 1; NS <= 16; ++NS) {
-            if (fNS && NS != fNS) continue;
-            const int spw = 32 / T;
-            int NT = (NS * nslots + spw - 1) / spw * 32;
-            int lanes = NS * ls;
-            if (NT > 1024) break;
-            if ((int64_t)NT * (2 * C + 40) > 65536) continue;   // register file (verified against the real kernel at configure time)
-            size_t smem = prof_bytes + (size_t)NS * ((size_t)max_seg_len + 64) + 256;
-            if (smem > kSmemLimit) continue;
-            (void)lanes;
-            double cost = geometry_cost(C, T, NS, NT, smem, std::max<int64_t>(nseg_hint, 1), std::max(max_seg_len, 1));
-            cost *= 1.0 + 0.002 * (NS - 1);           // ties: prefer fewer segments per CTA
-            if (cost < best) { best = cost; bestC = C; bestT = T; bestNS = NS; bestNT = NT; }
+    auto classic_search = [&](bool streamed) {
+        for (int C : kC) for (int T : kT) {
+            if (fC && (C != fC || T != fT)) continue;
+            if (C * T < ms.Lmax) continue;
+            if (!fC && C > 24 && !need_big) continue;
+            int ls = nslots * T;                        // lanes per segment
+            if (ls > 1024) continue;
+            const int qpc = ((C + 3) / 4) | 1;
+            size_t prof_bytes = (size_t)5 * qpc * ls * 16;
+            for (int NS = 1; NS <= 16; ++NS) {
+                if (fNS && NS != fNS) continue;
+                const int spw = 32 / T;
+                int NT = (NS * nslots + spw - 1) / spw * 32;
+                if (NT > 1024) break;
+                if ((int64_t)NT * (2 * C + 40) > 65536) continue;   // register file (verified against the real kernel at configure time)
+                size_t smem = prof_bytes + (streamed ? 0 : (size_t)NS * ((size_t)max_seg_len + 64)) + 256;
+                if (smem > kSmemLimit) continue;
+                double cost = geometry_cost(C, T, NS, NT, smem, std::max<int64_t>(nseg_hint, 1), std::max(max_seg_len, 1));
+                cost *= 1.0 + 0.002 * (NS - 1);           // ties: prefer fewer segments per CTA
+                if (cost < best) { best = cost; bestC = C; bestT = T; bestNS = NS; bestNT = NT; }
+            }
         }
-    }
+    };
+    classic_search(stream);
     Geometry &g = p.g;
     g.NG = 1;
     int force_sg = 0;
@@ -251,12 +256,16 @@ Plan make_plan(const MonomerSet &ms, const Scoring &sc, int max_seg_len, int64_t
             g.NG = ng;
             g.SG = sg;
         } else if (!bestC) {
-            throw PlanError{"internal: no launch geometry for this monomer set"};
+            // one group covers the set: only the segment length kept the symbols out of shared memory
+            classic_search(true);
+            if (!bestC) throw PlanError{"internal: no launch geometry for this monomer set"};
+            stream = 1;
         }                                    // a forced group size that covers every slot is the ordinary single-CTA sweep
     }
     g.packed = packed; g.C = bestC; g.T = bestT; g.nslots = nslots; g.M = ms.M; g.NS = bestNS; g.NT = bestNT;
     if (g.NG == 1) g.SG = nslots;
     g.lat = 0;
+    g.stream = g.NG > 1 ? 0 : stream;         // the group sweep always reads its symbols from global memory
     // Deferred-jump sweep (sweep_core.cuh: lat_*): a segment is spread over many warps -- a cluster of CTAs that exchange
     // the column key through distributed shared memory -- and runs at the latency of one column instead of at the
     // throughput of a loaded SM.  It pays when there are too few segments to fill the GPU with classic CTAs (config 1,
@@ -267,7 +276,8 @@ Plan make_plan(const MonomerSet &ms, const Scoring &sc, int max_seg_len, int64_t
         if (const char *e = getenv("SD_LAT_WARPS")) lat_warps = atoi(e);
         const int64_t nseg = std::max<int64_t>(nseg_hint, 1);
         double lbest = 1e300; int lC = 0, lT = 0, lNT = 0, lNG = 0, lSG = 0, lW = 0;
-        if (lat_mode != 0 && force_sg <= 0)
+        auto lat_search = [&](bool streamed) {
+            if (lat_mode == 0 || force_sg > 0) return;
             for (auto &cand : kLatGeom) {
                 const int C = cand[0], T = cand[1];
                 if (fC && (C != fC || T != fT)) continue;
@@ -283,7 +293,7 @@ Plan make_plan(const MonomerSet &ms, const Scoring &sc, int max_seg_len, int64_t
                 wc = (ws + (ws + wc - 1) / wc - 1) / ((ws + wc - 1) / wc);                    // even out the CTAs of a cluster
                 const int ng = (ws + wc - 1) / wc, sg = wc * spw;
                 const int qp2c = ((2 * C + 3) / 4) | 1;
-                const size_t smem = (size_t)5 * sg * T * qp2c * 16 + (size_t)max_seg_len + 4096;
+                const size_t smem = (size_t)5 * sg * T * qp2c * 16 + (streamed ? 0 : (size_t)max_seg_len) + 4096;
                 if (smem > kSmemLimit) continue;
                 // Measured on the B200 (tools/lat_probe.py, profiles/r02_lat_timing.txt, 12 DXZ1 monomers).  With one CTA
                 // per SM a column takes 415 cycles at (6,32), 510 at (12,16), 605 at (24,8); every further CTA that has
@@ -297,9 +307,15 @@ Plan make_plan(const MonomerSet &ms, const Scoring &sc, int max_seg_len, int64_t
                 const double cost = (double)std::max(max_seg_len, 1) * base * (1.0 + 0.3 * std::pow(C / 6.0, 0.6) * (ctas_sm - 1));
                 if (cost < lbest) { lbest = cost; lC = C; lT = T; lNT = wc * 32; lNG = ng; lSG = sg; lW = W; }
             }
+        };
+        // streamed candidates only where the classic sweep streams too, or where SD_LAT=1 finds no staged one
+        lat_search(stream);
+        int lstream = stream;
+        if (!lC && !stream && lat_mode > 0) { lat_search(true); lstream = 1; }
         const bool want = lat_mode > 0 || (lat_mode < 0 && lC && g.NG == 1 && nseg <= 2 * 148 && lbest < 0.97 * best);
         if (want && lC) {
             g.lat = 1; g.C = lC; g.T = lT; g.NS = 1; g.NT = lNT; g.NG = lNG; g.SG = lNG > 1 ? lSG : nslots; g.scanw = lW;
+            g.stream = lstream;
         } else if (lat_mode > 0) {
             throw PlanError{"SD_LAT=1: no deferred-jump geometry fits this monomer set"};
         }

@@ -334,6 +334,8 @@ struct Geometry {
     int SG;          // slots per group (== nslots when NG == 1)
     int lat;         // 1: deferred-jump sweep (sweep_lat_kernel; a segment = a cluster of NG CTAs, NS == 1), 0: classic
     int scanw;       // lanes a lane must look back for the deletion carry (windowed scan; see plan.cpp: scan_window)
+    int stream;      // 1: the classic / deferred-jump sweep reads the segment symbols from global memory as it goes
+                     // (shared memory independent of the segment length); 0: they are staged in shared memory first
 };
 
 struct Record { int32_t row, start, end, score; };

@@ -1,5 +1,5 @@
 // instantiations of sweep_kernel<Scalar32, C, T, FAST=1, MULTI=0>
 #include "sweep_kernel.cuh"
 namespace sdb {
-SD_INSTANTIATE_SWEEP(sweep_lookup_s32_f1_m0, Scalar32, true, false)
+SD_INSTANTIATE_SWEEP(sweep_lookup_s32_f1_m0, Scalar32, true, false, false)
 }

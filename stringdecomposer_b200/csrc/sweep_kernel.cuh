@@ -59,7 +59,10 @@ __device__ __forceinline__ uint32_t slot_scan_window(uint32_t E, int t, uint32_t
 // reduced with CREDUX inside the warp and exchanged through one aligned int4 row of shared memory.
 // MULTI (with FAST): several segments share the CTA and its profile table but synchronise separately (named barriers).
 // !FAST: arbitrary lane->segment mapping; keys meet in shared-memory atomicMax (three rotating buffers).
-template <class P, int C, int T, bool FAST, bool MULTI>
+// STREAM: the segment symbols are not staged in shared memory (whose size then does not depend on the segment length):
+// every thread loads the symbol of column i+2 from global memory while it sweeps column i, the same symbol for all
+// lanes of a segment (one L1 broadcast), and validates and encodes it as the staging loop does.
+template <class P, int C, int T, bool FAST, bool MULTI, bool STREAM = false>
 __device__ __forceinline__ void sweep_body(const SweepArgs &a)
 {
     extern __shared__ uint4 smem_u4[];
@@ -86,7 +89,7 @@ __device__ __forceinline__ void sweep_body(const SweepArgs &a)
 
     // stage profile, segment symbols and keys
     for (int x = tid; x < a.prof_u4; x += NT) sprof[x] = a.prof[x];
-    for (int s = 0; s < NS; ++s) {
+    for (int s = 0; s < (STREAM ? 0 : NS); ++s) {
         int n = 0; const uint8_t *src = nullptr;
         if (first + s < a.nseg) {
             const int64_t o = a.seg_off[first + s];
@@ -121,6 +124,13 @@ __device__ __forceinline__ void sweep_body(const SweepArgs &a)
     uint32_t *cptr = a.codes + a.cta_code_off[cta] + (size_t)tid * a.CW;
     const size_t cstride = (size_t)NT * a.CW;
     const uint8_t *cp = schar + seg_local * a.seg_stride;               // symbol of the column being prepared
+    // STREAM: the segment's text in global memory; columns past its end read as symbol 0, like the 0-padded buffer
+    const uint8_t *src = a.bases + (active ? a.seg_off[first + seg_local] : 0);
+    auto symbol = [&](int i) {
+        int code = (i < n_seg) ? ascii_code(__ldg(src + i)) : 0;
+        if (code > 4) { *a.bad_symbol = 1; code = 0; }
+        return code;
+    };
     const uint4 *myprof = sprof + (size_t)(slot * T + t) * a.qp;
     const int sym_stride = a.nsl * a.qp;
     // FAST: segment s of the CTA owns int4 row s of each key buffer, its warps write one int each.  Raw shared-space
@@ -147,7 +157,9 @@ __device__ __forceinline__ void sweep_body(const SweepArgs &a)
 
     // column 0: everything dead, base B[0] = ins (row-0 rule, main.cpp:180); the k==0 cell is s(0,0) itself
     // (main.cpp:173-177), i.e. one `del` more than the generic jump candidate
-    load_profile(*cp++);
+    int sym_next = 0;
+    if (STREAM) { load_profile(symbol(0)); sym_next = symbol(1); }
+    else load_profile(*cp++);
     if (t == 0 && L > 1) pw[0] = P::add(pw[0], P::splat(4 * a.del));
     if (t == T - 1 && L == 1) pw[C - 1] = P::add(pw[C - 1], P::splat(4 * a.del));
     lane_pre<P, C>(X, deadu, pw, deadu, kill_first, kill_last);
@@ -159,7 +171,8 @@ __device__ __forceinline__ void sweep_body(const SweepArgs &a)
         const uint32_t E = lane_post<P, C>(X, pw, P::splat(jump0 + 1), deadu, tr);
         // profile of the next column (the symbol buffer is 0-padded, so the round after the last column is harmless);
         // issued here so that the loads fly during the scan
-        load_profile(*cp++);
+        if (STREAM) { load_profile(sym_next); sym_next = symbol(i + 2); }
+        else load_profile(*cp++);
         const uint32_t carry = slot_scan_window<P, T>(E, t, deadu, a.scanw);
         constexpr int NW = (C + P::CELLS_PER_WORD - 1) / P::CELLS_PER_WORD;
         uint32_t cw[NW];
@@ -234,14 +247,14 @@ __device__ __forceinline__ void sweep_body(const SweepArgs &a)
 }
 
 
-template <class P, int C, int T, bool FAST, bool MULTI>
-__global__ void sweep_kernel(const SweepArgs a) { sweep_body<P, C, T, FAST, MULTI>(a); }
+template <class P, int C, int T, bool FAST, bool MULTI, bool STREAM>
+__global__ void sweep_kernel(const SweepArgs a) { sweep_body<P, C, T, FAST, MULTI, STREAM>(a); }
 
 // The same kernel with its register budget pinned at 80: saturated launches (several segments per CTA, C <= 24) then fit
 // two 384-thread CTAs per SM; left alone ptxas settles on 96 registers and halves the occupancy (measured: 3.95 -> 4.11
 // TCUPS on 4,000 segments).  Only used for CTAs of at most 768 threads.
-template <class P, int C, int T, bool FAST, bool MULTI>
-__global__ void __maxnreg__(80) sweep_kernel_r80(const SweepArgs a) { sweep_body<P, C, T, FAST, MULTI>(a); }
+template <class P, int C, int T, bool FAST, bool MULTI, bool STREAM>
+__global__ void __maxnreg__(80) sweep_kernel_r80(const SweepArgs a) { sweep_body<P, C, T, FAST, MULTI, STREAM>(a); }
 
 // ---------------------------------------------------------------------------------------------------------------
 // Group sweep: monomer sets that do not fit one CTA (threads, registers, or the shared-memory profile table).
@@ -442,35 +455,41 @@ __global__ void sweep_group_kernel(const GroupArgs a)
     }
 }
 
-// lookup tables of the instantiations, one translation unit per (policy, FAST, MULTI) so that they build in parallel
+// lookup tables of the instantiations, one translation unit per (policy, FAST, MULTI, STREAM) so that they build in parallel
 const void *sweep_lookup_p16_f1_m0(int C, int T, int NT);
 const void *sweep_lookup_p16_f1_m1(int C, int T, int NT);
 const void *sweep_lookup_p16_f0_m0(int C, int T, int NT);
 const void *sweep_lookup_s32_f1_m0(int C, int T, int NT);
 const void *sweep_lookup_s32_f1_m1(int C, int T, int NT);
 const void *sweep_lookup_s32_f0_m0(int C, int T, int NT);
+const void *sweep_lookup_p16_f1_m0_st(int C, int T, int NT);
+const void *sweep_lookup_p16_f1_m1_st(int C, int T, int NT);
+const void *sweep_lookup_p16_f0_m0_st(int C, int T, int NT);
+const void *sweep_lookup_s32_f1_m0_st(int C, int T, int NT);
+const void *sweep_lookup_s32_f1_m1_st(int C, int T, int NT);
+const void *sweep_lookup_s32_f0_m0_st(int C, int T, int NT);
 const void *sweep_group_lookup_p16(int C, int T);
 const void *sweep_group_lookup_s32(int C, int T);
 
 // the register-capped twin is instantiated only where it is used: several segments per CTA (LL) and C <= 24
-template <class POLICY, int CC, int TT, bool FAST, bool LL> static const void *sweep_pick(bool cap80)
+template <class POLICY, int CC, int TT, bool FAST, bool LL, bool ST> static const void *sweep_pick(bool cap80)
 {
-    if constexpr (LL && CC <= 24) { if (cap80) return (const void *)sweep_kernel_r80<POLICY, CC, TT, FAST, LL>; }
+    if constexpr (LL && CC <= 24) { if (cap80) return (const void *)sweep_kernel_r80<POLICY, CC, TT, FAST, LL, ST>; }
     (void)cap80;
-    return (const void *)sweep_kernel<POLICY, CC, TT, FAST, LL>;
+    return (const void *)sweep_kernel<POLICY, CC, TT, FAST, LL, ST>;
 }
-#define SD_SWEEP_PICK(POLICY, CC, TT, FAST, LL) sweep_pick<POLICY, CC, TT, FAST, LL>(cap80)
-#define SD_INSTANTIATE_SWEEP(NAME, POLICY, FAST, LL)                                                                 \
+#define SD_SWEEP_PICK(POLICY, CC, TT, FAST, LL, ST) sweep_pick<POLICY, CC, TT, FAST, LL, ST>(cap80)
+#define SD_INSTANTIATE_SWEEP(NAME, POLICY, FAST, LL, ST)                                                             \
     template <int C> static const void *NAME##_t(int T, bool cap80)                                                  \
     {                                                                                                                 \
         switch (T) {                                                                                                  \
-        case 1: return SD_SWEEP_PICK(POLICY, C, 1, FAST, LL);                                                         \
-        case 2: return SD_SWEEP_PICK(POLICY, C, 2, FAST, LL);                                                         \
-        case 4: return SD_SWEEP_PICK(POLICY, C, 4, FAST, LL);                                                         \
-        case 8: return SD_SWEEP_PICK(POLICY, C, 8, FAST, LL);                                                         \
-        case 10: return SD_SWEEP_PICK(POLICY, C, 10, FAST, LL);                                                       \
-        case 16: return SD_SWEEP_PICK(POLICY, C, 16, FAST, LL);                                                       \
-        case 32: return SD_SWEEP_PICK(POLICY, C, 32, FAST, LL);                                                       \
+        case 1: return SD_SWEEP_PICK(POLICY, C, 1, FAST, LL, ST);                                                     \
+        case 2: return SD_SWEEP_PICK(POLICY, C, 2, FAST, LL, ST);                                                     \
+        case 4: return SD_SWEEP_PICK(POLICY, C, 4, FAST, LL, ST);                                                     \
+        case 8: return SD_SWEEP_PICK(POLICY, C, 8, FAST, LL, ST);                                                     \
+        case 10: return SD_SWEEP_PICK(POLICY, C, 10, FAST, LL, ST);                                                   \
+        case 16: return SD_SWEEP_PICK(POLICY, C, 16, FAST, LL, ST);                                                   \
+        case 32: return SD_SWEEP_PICK(POLICY, C, 32, FAST, LL, ST);                                                   \
         }                                                                                                             \
         return nullptr;                                                                                               \
     }                                                                                                                 \

@@ -218,23 +218,23 @@ __global__ void hw_distance_kernel(const uint8_t *bases, const int64_t *seg_off,
 }
 
 // The same for rows of at most 64*NB symbols (NB <= 4: alpha-satellite monomers need 3): a CTA takes one segment and 128
-// rows, one row per thread.  The segment's symbols are staged in shared memory once and broadcast; the match masks of the
-// CTA's rows live in shared memory as [symbol][word][thread] (conflict-free 8-byte loads); the Myers/Hyyro column state
-// stays in registers.  Same recurrence as sweep_core.cuh: hw_distance (edlib's HW mode, distance only).
+// rows, one row per thread.  The segment's symbols pass through shared memory in tiles of HWF_TILE (one barrier per tile,
+// so a segment of any length fits) and are broadcast; the match masks of the CTA's rows live in shared memory as
+// [symbol][word][thread] (conflict-free 8-byte loads); the Myers/Hyyro column state stays in registers.  Same recurrence
+// as sweep_core.cuh: hw_distance (edlib's HW mode, distance only).
 constexpr int HWF_ROWS = 128;
+constexpr int HWF_TILE = 4096;
 template <int NB>
 __global__ void __launch_bounds__(HWF_ROWS) hw_distance_rows_kernel(const uint8_t *bases, const int64_t *seg_off, const uint8_t *rows,
-                                                                    const int *row_off, int R, int *dist, int text_stride)
+                                                                    const int *row_off, int R, int *dist)
 {
     extern __shared__ unsigned long long hwf_smem[];
     unsigned long long *peq = hwf_smem;                                  // [5][NB][HWF_ROWS]
-    uint8_t *stext = reinterpret_cast<uint8_t *>(peq + 5 * NB * HWF_ROWS);
+    uint8_t *stext = reinterpret_cast<uint8_t *>(peq + 5 * NB * HWF_ROWS);     // [HWF_TILE]
     const int s = blockIdx.x, tid = threadIdx.x;
     const int r = blockIdx.y * HWF_ROWS + tid;
     const int64_t o = seg_off[s];
     const int n = (int)(seg_off[s + 1] - o);
-    (void)text_stride;
-    for (int x = tid; x < n; x += HWF_ROWS) { const int c = ascii_code(bases[o + x]); stext[x] = (uint8_t)(c > 4 ? 4 : c); }
 #pragma unroll
     for (int q = 0; q < 5 * NB; ++q) peq[q * HWF_ROWS + tid] = 0ull;
     int m = 0;
@@ -247,40 +247,45 @@ __global__ void __launch_bounds__(HWF_ROWS) hw_distance_rows_kernel(const uint8_
             peq[(c * NB + (i >> 6)) * HWF_ROWS + tid] |= 1ull << (i & 63);
         }
     }
-    __syncthreads();
-    if (r >= R) return;
     const int B = (m + 63) >> 6;
     unsigned long long pv[NB], mv[NB];
 #pragma unroll
     for (int b = 0; b < NB; ++b) { pv[b] = ~0ull; mv[b] = 0ull; }
     const unsigned long long last_bit = 1ull << ((m - 1) & 63);
     int score = m, best = m;
-    for (int j = 0; j < n; ++j) {
-        const int c = stext[j];
-        int hin = 0;
+    for (int j0 = 0; j0 < n; j0 += HWF_TILE) {
+        const int len = min(HWF_TILE, n - j0);
+        __syncthreads();                                                  // the previous tile is consumed (first: peq is built)
+        for (int x = tid; x < len; x += HWF_ROWS) { const int c = ascii_code(bases[o + j0 + x]); stext[x] = (uint8_t)(c > 4 ? 4 : c); }
+        __syncthreads();
+        if (r >= R) continue;
+        for (int j = 0; j < len; ++j) {
+            const int c = stext[j];
+            int hin = 0;
 #pragma unroll
-        for (int b = 0; b < NB; ++b) {
-            if (b < B) {
-                unsigned long long eq = peq[(c * NB + b) * HWF_ROWS + tid];
-                const unsigned long long p = pv[b], mm = mv[b];
-                const unsigned long long xv = eq | mm;
-                if (hin < 0) eq |= 1ull;
-                const unsigned long long xh = (((eq & p) + p) ^ p) | eq;
-                unsigned long long ph = mm | ~(xh | p);
-                unsigned long long mh = p & xh;
-                const unsigned long long top = (b == B - 1) ? last_bit : (1ull << 63);
-                const int hout = (ph & top) ? 1 : ((mh & top) ? -1 : 0);
-                ph <<= 1; mh <<= 1;
-                if (hin < 0) mh |= 1ull; else if (hin > 0) ph |= 1ull;
-                pv[b] = mh | ~(xv | ph);
-                mv[b] = ph & xv;
-                hin = hout;
+            for (int b = 0; b < NB; ++b) {
+                if (b < B) {
+                    unsigned long long eq = peq[(c * NB + b) * HWF_ROWS + tid];
+                    const unsigned long long p = pv[b], mm = mv[b];
+                    const unsigned long long xv = eq | mm;
+                    if (hin < 0) eq |= 1ull;
+                    const unsigned long long xh = (((eq & p) + p) ^ p) | eq;
+                    unsigned long long ph = mm | ~(xh | p);
+                    unsigned long long mh = p & xh;
+                    const unsigned long long top = (b == B - 1) ? last_bit : (1ull << 63);
+                    const int hout = (ph & top) ? 1 : ((mh & top) ? -1 : 0);
+                    ph <<= 1; mh <<= 1;
+                    if (hin < 0) mh |= 1ull; else if (hin > 0) ph |= 1ull;
+                    pv[b] = mh | ~(xv | ph);
+                    mv[b] = ph & xv;
+                    hin = hout;
+                }
             }
+            score += hin;
+            best = min(best, score);
         }
-        score += hin;
-        best = min(best, score);
     }
-    dist[(size_t)s * R + r] = best;
+    if (r < R) dist[(size_t)s * R + r] = best;
 }
 
 // Step 2: per segment, the rows sorted by (distance, row); the closest row and every row within ed_thr are kept
@@ -376,8 +381,12 @@ template <int MODE> __global__ void int_peak_kernel(unsigned *out, unsigned seed
 }
 
 // ---------------------------------------------------------------------------------------------
-static const void *kern(int packed, int C, int T, int NT, bool fast, bool multi)
+static const void *kern(int packed, int C, int T, int NT, bool fast, bool multi, bool stream)
 {
+    if (stream) {
+        if (packed) return fast ? (multi ? sweep_lookup_p16_f1_m1_st(C, T, NT) : sweep_lookup_p16_f1_m0_st(C, T, NT)) : sweep_lookup_p16_f0_m0_st(C, T, NT);
+        return fast ? (multi ? sweep_lookup_s32_f1_m1_st(C, T, NT) : sweep_lookup_s32_f1_m0_st(C, T, NT)) : sweep_lookup_s32_f0_m0_st(C, T, NT);
+    }
     if (packed) return fast ? (multi ? sweep_lookup_p16_f1_m1(C, T, NT) : sweep_lookup_p16_f1_m0(C, T, NT)) : sweep_lookup_p16_f0_m0(C, T, NT);
     return fast ? (multi ? sweep_lookup_s32_f1_m1(C, T, NT) : sweep_lookup_s32_f1_m0(C, T, NT)) : sweep_lookup_s32_f0_m0(C, T, NT);
 }
@@ -483,6 +492,7 @@ public:
         if (prop_.major != 10) throw PlanError{"CUDA device is not sm_100 class: this library carries sm_100a code only (no PTX for other architectures)"};
         size_t fr = 0, tot = 0;
         SD_CUDA(cudaMemGetInfo(&fr, &tot));
+        free_at_start_ = (int64_t)fr;
         budget_ = std::min<int64_t>((int64_t)(fr * 0.85), (int64_t)96 << 30);
     }
     ~CudaBackend() override
@@ -506,12 +516,13 @@ public:
         if (getenv("SD_NOFAST")) fast_ = false;
         lat_timing_ = false;
         if (g.lat) {
-            kernel_ = g.packed ? sweep_lat_lookup_p16(g.C, g.T, g.scanw) : sweep_lat_lookup_s32(g.C, g.T, g.scanw);
-            if (getenv("SD_LAT_TIMING") && g.packed && sweep_lat_timing_lookup_p16(g.C, g.T, g.scanw)) { kernel_ = sweep_lat_timing_lookup_p16(g.C, g.T, g.scanw); lat_timing_ = true; }
+            if (g.stream) kernel_ = g.packed ? sweep_lat_lookup_p16_st(g.C, g.T, g.scanw) : sweep_lat_lookup_s32_st(g.C, g.T, g.scanw);
+            else kernel_ = g.packed ? sweep_lat_lookup_p16(g.C, g.T, g.scanw) : sweep_lat_lookup_s32(g.C, g.T, g.scanw);
+            if (getenv("SD_LAT_TIMING") && g.packed && !g.stream && sweep_lat_timing_lookup_p16(g.C, g.T, g.scanw)) { kernel_ = sweep_lat_timing_lookup_p16(g.C, g.T, g.scanw); lat_timing_ = true; }
             if ((g.NT / 32) * g.NG > 32) throw PlanError{"internal: a deferred-jump cluster holds at most 32 warps"};
         }
         else kernel_ = g.NG > 1 ? (g.packed ? sweep_group_lookup_p16(g.C, g.T) : sweep_group_lookup_s32(g.C, g.T))
-                                : kern(g.packed, g.C, g.T, g.NT, fast_, fast_ && g.NS > 1);
+                                : kern(g.packed, g.C, g.T, g.NT, fast_, fast_ && g.NS > 1, g.stream != 0);
         if (!kernel_) throw PlanError{"no sweep kernel compiled for this geometry"};
         cudaFuncAttributes fa;
         SD_CUDA(cudaFuncGetAttributes(&fa, kernel_));
@@ -559,6 +570,7 @@ public:
         if (const char *e = getenv("SD_WAVE_BYTES")) if (atoll(e) > 0) return atoll(e);
         return budget_;        // 85 % of the memory that was free when the backend was created (cudaMemGetInfo costs ms)
     }
+    int64_t device_bytes() const override { return free_at_start_; }
     int wave_slots() const override { return 2; }
 
     // Buffers of a slot sized for the largest wave it will see: growing them later would mean cudaFree (a device-wide
@@ -627,16 +639,14 @@ public:
         w.d_dist.need(np * 4); w.d_rank.need(np * 4); w.d_r2r.need(np * 4);
         const int NB = (ms_.Lmax + 63) / 64;
         if (NB <= 4) {
-            const int text_stride = (w.nmax + 16) / 16 * 16;
-            const size_t smem = (size_t)5 * NB * HWF_ROWS * 8 + (size_t)text_stride;
+            const size_t smem = (size_t)5 * NB * HWF_ROWS * 8 + (size_t)std::min(HWF_TILE, (w.nmax + 16) / 16 * 16);
             const void *k = NB == 1 ? (const void *)hw_distance_rows_kernel<1> : NB == 2 ? (const void *)hw_distance_rows_kernel<2>
                           : NB == 3 ? (const void *)hw_distance_rows_kernel<3> : (const void *)hw_distance_rows_kernel<4>;
-            if (smem > (size_t)prop_.sharedMemPerBlockOptin) throw PlanError{"--ed_thr: segment too long for the pre-filter kernel"};
             SD_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             const uint8_t *bases = w.d_bases.as<uint8_t>(); const int64_t *so = w.d_segoff.as<int64_t>();
             const uint8_t *rows = d_rows_.as<uint8_t>(); const int *ro = d_rowoff_.as<int>(); int *dist = w.d_dist.as<int>();
-            int Rv = R, ts = text_stride;
-            void *args[] = {(void *)&bases, (void *)&so, (void *)&rows, (void *)&ro, (void *)&Rv, (void *)&dist, (void *)&ts};
+            int Rv = R;
+            void *args[] = {(void *)&bases, (void *)&so, (void *)&rows, (void *)&ro, (void *)&Rv, (void *)&dist};
             SD_CUDA(cudaLaunchKernel(k, dim3((unsigned)w.nseg, (unsigned)((R + HWF_ROWS - 1) / HWF_ROWS)), dim3(HWF_ROWS), args, smem, st_in_));
         } else {
             hw_distance_kernel<<<(unsigned)((np + 63) / 64), 64, 0, st_in_>>>(w.d_bases.as<uint8_t>(), w.d_segoff.as<int64_t>(), w.nseg,
@@ -672,7 +682,7 @@ public:
         a.kstride = fast_ ? g.NS * 4 : (g.NS + 3) / 4 * 4;
         a.tr = g.packed ? tag_regs<Packed16>() : tag_regs<Scalar32>();
         a.scanw = getenv("SD_FULL_SCAN") ? 64 : g.scanw;
-        const size_t smem = plan_.prof.size() * 4 + (size_t)3 * a.kstride * 4 + (size_t)g.NS * a.seg_stride;
+        const size_t smem = plan_.prof.size() * 4 + (size_t)3 * a.kstride * 4 + (g.stream ? 0 : (size_t)g.NS * a.seg_stride);
         if (smem > (size_t)prop_.sharedMemPerBlockOptin) throw PlanError{"sweep geometry needs more shared memory than the SM has"};
         SD_CUDA(cudaFuncSetAttribute(kernel_, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         const int nctas = (int)w.lay.cta_nmax.size();
@@ -735,7 +745,7 @@ public:
         a.dbg = nullptr;
         if (lat_timing_) { w.d_dbg.need((size_t)w.nseg * g.NG * wpc * 64); a.dbg = w.d_dbg.as<long long>(); SD_CUDA(cudaMemsetAsync(a.dbg, 0, (size_t)w.nseg * g.NG * wpc * 64, st_)); }
         const size_t sgt = (size_t)wpc * spw * g.T;
-        const size_t smem = (size_t)5 * sgt * plan_.qp2 * 16 + (size_t)LAT_NBUF * 32 * 8 + 32 + (size_t)seg_stride;
+        const size_t smem = (size_t)5 * sgt * plan_.qp2 * 16 + (size_t)LAT_NBUF * 32 * 8 + 32 + (g.stream ? 0 : (size_t)seg_stride);
         if (smem > (size_t)prop_.sharedMemPerBlockOptin) throw PlanError{"deferred-jump sweep needs more shared memory than the SM has"};
         SD_CUDA(cudaFuncSetAttribute(kernel_, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         cudaLaunchConfig_t cfg{};
@@ -929,6 +939,7 @@ private:
     bool fast_ = false, lat_timing_ = false;
     std::vector<uint8_t> rows_ascii_;
     int64_t budget_ = 0;
+    int64_t free_at_start_ = 0;        // device memory that was free when the backend was created
     DevBuf d_prof_, d_slotlen_, d_slotend_, d_rows_, d_rowoff_, d_kjbase_;
     std::vector<int> kjbase_;
     WaveSlot slot_[2];

@@ -84,7 +84,10 @@ __device__ __forceinline__ uint32_t window_carry(uint32_t total, int t, uint32_t
     return pv;
 }
 
-template <class P, int C, int T, int WN, bool TM = false>
+// ST: the segment symbols are not staged in shared memory (whose size then does not depend on the segment length):
+// every thread loads the symbol of column i+2 from global memory while it sweeps column i (one L1 broadcast per warp);
+// column i uses the symbol of column i+1 for its look-ahead profile load, so the load has a whole column to land.
+template <class P, int C, int T, int WN, bool TM = false, bool ST = false>
 __global__ void sweep_lat_kernel(const LatArgs a)
 {
     extern __shared__ uint4 smem_u4[];
@@ -117,7 +120,7 @@ __global__ void sweep_lat_kernel(const LatArgs a)
         const int row = min((NG > 1 ? grp * a.SG * T : 0) + r / a.qp2, a.nsl_total - 1);
         sprof[x] = a.prof2[((size_t)sym * a.nsl_total + row) * a.qp2 + (r % a.qp2)];
     }
-    for (int x = tid; x < a.seg_stride; x += NT) {
+    for (int x = tid; x < (ST ? 0 : a.seg_stride); x += NT) {
         int code = (x < n) ? ascii_code(a.bases[o + x]) : 0;
         if (code > 4) { *a.bad_symbol = 1; code = 0; }
         schar[x] = (uint8_t)code;
@@ -229,17 +232,24 @@ __global__ void sweep_lat_kernel(const LatArgs a)
         cptr += cstride;
     };
 
+    // ST: symbols past the end of the segment read as 0, like the 0-padded buffer
+    auto symbol = [&](int i) {
+        int code = (i < n) ? ascii_code(__ldg(a.bases + o + i)) : 0;
+        if (code > 4) { *a.bad_symbol = 1; code = 0; }
+        return code;
+    };
+
     // ---- column 0 in the classic form: its jump base (row-0 rule, main.cpp:171-182) needs no exchange -------------
 #pragma unroll
     for (int kk = 0; kk < C; ++kk) X[kk] = deadu;
-    load_p(myprof + schar[0] * sym_stride);
+    load_p(myprof + (ST ? symbol(0) : schar[0]) * sym_stride);
     if (t == 0 && L > 1) pw[0] = P::add(pw[0], P::splat(4 * a.del));
     if (t == T - 1 && L == 1) pw[C - 1] = P::add(pw[C - 1], P::splat(4 * a.del));
     lane_pre<P, C>(X, deadu, pw, deadu, kill_first, kill_last);
     {
         const uint32_t E = lane_post<P, C>(X, pw, P::splat(1), deadu, tr);
         const uint32_t carry = window_carry<P, T, 0>(E, t, deadu);
-        const uint32_t pn = myprof + schar[1] * sym_stride;
+        const uint32_t pn = myprof + (ST ? symbol(1) : schar[1]) * sym_stride;
         load_p(pn);
         load_pt(pn);
         uint32_t ufirst;
@@ -271,13 +281,15 @@ __global__ void sweep_lat_kernel(const LatArgs a)
     auto tick = [&](int ph) { if (TM) { const long long c = clock64(); tacc[ph] += c - tprev; tprev = c; } };
     if (TM) tprev = clock64();
     const uint8_t *sp = schar + 2;
-    int sym = schar[1];
+    int sym = ST ? symbol(1) : schar[1];
+    int sym_ahead = ST ? symbol(2) : 0;       // ST: symbol of column i+1, loaded one column before it is needed
     uint32_t boff = 256u, boff_prev = 0u;                  // 256 * (i & 3), 256 * ((i-1) & 3)
 #pragma unroll 1
     for (int i = 1; i < n; ++i, ++sp) {
         // J-independent part of column i (X holds max(diag, up))
         const uint32_t total = lat_total<P, C>(X, trr);
-        const int symn = sp[0];
+        const int symn = ST ? sym_ahead : sp[0];
+        if (ST) sym_ahead = symbol(i + 2);
         const uint32_t pn = myprof + (uint32_t)symn * sym_stride;
         const uint32_t carry = window_carry<P, T, WN>(total, t, deadu);
         tick(0);
@@ -342,23 +354,26 @@ __global__ void sweep_lat_kernel(const LatArgs a)
 // WN: carry window the kernel is compiled for (0 = any, log-depth scan)
 const void *sweep_lat_lookup_p16(int C, int T, int W);
 const void *sweep_lat_lookup_s32(int C, int T, int W);
+const void *sweep_lat_lookup_p16_st(int C, int T, int W);                 // ST: symbols streamed from global memory
+const void *sweep_lat_lookup_s32_st(int C, int T, int W);
 const void *sweep_lat_timing_lookup_p16(int C, int T, int W);            // instrumented twins (SD_LAT_TIMING=1, exploration only)
 
 // smallest compiled window >= W
-#define SD_LAT_PICK(POLICY, CC, TT, TMF)                                                                             \
+#define SD_LAT_PICK(POLICY, CC, TT, TMF, STF)                                                                        \
     if (C == CC && T == TT) {                                                                                         \
-        if (W <= 2) return (const void *)sweep_lat_kernel<POLICY, CC, TT, 2, TMF>;                                    \
-        if (W <= 4) return (const void *)sweep_lat_kernel<POLICY, CC, TT, 4, TMF>;                                    \
-        if (W <= 8) return (const void *)sweep_lat_kernel<POLICY, CC, TT, 8, TMF>;                                    \
-        return (const void *)sweep_lat_kernel<POLICY, CC, TT, 0, TMF>;                                                \
+        if (W <= 2) return (const void *)sweep_lat_kernel<POLICY, CC, TT, 2, TMF, STF>;                               \
+        if (W <= 4) return (const void *)sweep_lat_kernel<POLICY, CC, TT, 4, TMF, STF>;                               \
+        if (W <= 8) return (const void *)sweep_lat_kernel<POLICY, CC, TT, 8, TMF, STF>;                               \
+        return (const void *)sweep_lat_kernel<POLICY, CC, TT, 0, TMF, STF>;                                           \
     }
 
-#define SD_INSTANTIATE_LAT(NAME, POLICY)                                                                             \
+#define SD_INSTANTIATE_LAT(NAME, POLICY, STF)                                                                        \
     const void *NAME(int C, int T, int W)                                                                             \
     {                                                                                                                 \
-        SD_LAT_PICK(POLICY, 6, 32, false) SD_LAT_PICK(POLICY, 12, 16, false) SD_LAT_PICK(POLICY, 12, 32, false)       \
-        SD_LAT_PICK(POLICY, 24, 8, false) SD_LAT_PICK(POLICY, 24, 16, false) SD_LAT_PICK(POLICY, 24, 32, false)       \
-        SD_LAT_PICK(POLICY, 48, 32, false)                                                                            \
+        SD_LAT_PICK(POLICY, 6, 32, false, STF) SD_LAT_PICK(POLICY, 12, 16, false, STF)                                \
+        SD_LAT_PICK(POLICY, 12, 32, false, STF) SD_LAT_PICK(POLICY, 24, 8, false, STF)                                \
+        SD_LAT_PICK(POLICY, 24, 16, false, STF) SD_LAT_PICK(POLICY, 24, 32, false, STF)                               \
+        SD_LAT_PICK(POLICY, 48, 32, false, STF)                                                                       \
         return nullptr;                                                                                               \
     }
 
