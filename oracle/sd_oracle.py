@@ -35,6 +35,8 @@ def lib():
         _lib.sdo_segment_read.restype = C.c_int
         _lib.sdo_postprocess.argtypes = [C.POINTER(Rec), C.c_int, C.POINTER(Rec)]
         _lib.sdo_postprocess.restype = C.c_int
+        _lib.sdo_filter_rows.argtypes = [C.c_char_p, C.c_int, C.c_char_p, C.POINTER(C.c_int), C.c_int, C.c_int, C.POINTER(C.c_int)]
+        _lib.sdo_filter_rows.restype = C.c_int
     return _lib
 
 
@@ -46,9 +48,24 @@ def rows_of(monomers):
     return list(monomers) + ["".join(_COMP[c] for c in reversed(m)) for m in monomers]
 
 
-def align_segment(seg, monomers, scoring=(-1, -1, -1, 1)):
-    """AlignPartClassicDP on one segment -> list of (row, start, end, score)"""
+def filter_rows(seg, rows, ed_thr):
+    """FilterMonomersForRead (main.cpp:135-149): indices of the rows kept for `seg`, in their new order"""
+    off = (C.c_int * (len(rows) + 1))()
+    for i, r in enumerate(rows):
+        off[i + 1] = off[i] + len(r)
+    keep = (C.c_int * max(len(rows), 1))()
+    n = lib().sdo_filter_rows(seg.encode(), len(seg), "".join(rows).encode(), off, len(rows), ed_thr, keep)
+    return [keep[i] for i in range(n)]
+
+
+def align_segment(seg, monomers, scoring=(-1, -1, -1, 1), ed_thr=-1):
+    """AlignPartClassicDP on one segment -> list of (row, start, end, score); ed_thr > -1 runs the rows that
+    FilterMonomersForRead keeps, with any scoring (the dp command line only combines --ed_thr with the default one)"""
     rows = rows_of(monomers)
+    keep = list(range(len(rows)))
+    if ed_thr > -1:
+        keep = filter_rows(seg, rows, ed_thr)
+        rows = [rows[k] for k in keep]
     off = (C.c_int * (len(rows) + 1))()
     for i, r in enumerate(rows):
         off[i + 1] = off[i] + len(r)
@@ -57,7 +74,7 @@ def align_segment(seg, monomers, scoring=(-1, -1, -1, 1)):
                                 scoring[2], scoring[3], out, len(seg) + 1)
     if n < 0:
         raise RuntimeError("oracle failed (%d)" % n)
-    return [(out[i].row, out[i].start, out[i].end, out[i].score) for i in range(n)]
+    return [(keep[out[i].row], out[i].start, out[i].end, out[i].score) for i in range(n)]
 
 
 def segment_read(read_len, part, overlap):

@@ -82,6 +82,7 @@ static int to_batch(const char *segments, const int64_t *offsets, int64_t n, Bat
 static int status_of(const std::string &msg)
 {
     if (msg.find("symbol outside") != std::string::npos) return SD_ERR_INPUT;
+    if (msg.rfind("internal error:", 0) == 0) return SD_ERR_INTERNAL;
     if (msg.find("CUDA") != std::string::npos) return SD_ERR_CUDA;
     return SD_ERR_UNSUPPORTED;
 }

@@ -69,6 +69,9 @@ struct BatchResult {
 };
 
 struct PlanError { std::string msg; };
+// A traceback met a jump row outside the DP rows (a wrong column key).  The C ABI reports messages that start with
+// "internal error:" as SD_ERR_INTERNAL.
+constexpr const char *SD_MSG_TB_BAD_ROW = "internal error: the traceback met a jump to a row outside the monomer set";
 
 // plan.cpp
 void build_monomer_set(const std::vector<std::string> &forward, MonomerSet &ms);     // throws PlanError

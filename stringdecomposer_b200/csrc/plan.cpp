@@ -104,6 +104,10 @@ void lat_jump_keys(const MonomerSet &ms, const Scoring &sc, const int *rank_of_r
 int scan_window(const MonomerSet &ms, const Scoring &sc, int packed, int C, int T)
 {
     if (T <= 1) return 0;
+    // In column 0 the first cell of a row is s(0,0) itself, one `del` above the jump candidate of its class
+    // (main.cpp:173-177).  With a positive deletion score it can beat every candidate of the slot, so every lane needs
+    // the total of lane 0.
+    if (sc.del > 0) return T - 1;
     const int nslots = packed ? ms.M : 2 * ms.M;
     const int SL = C * T;
     int W = 1;

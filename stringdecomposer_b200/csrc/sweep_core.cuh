@@ -23,6 +23,7 @@
 //   LOP3       U = (h | 3) ^ 1                   re-tag
 // and on the FMA pipe IMAD + IMAD.IADD for the backpointer digits w = w*4 + U - h.
 #pragma once
+#include <climits>
 #include <stdint.h>
 
 #if defined(__CUDACC__)
@@ -313,11 +314,42 @@ SD_HD int make_key(int z_end, int endadd, int row) { return ((z_end >> 2) + enda
 SD_HD int key_const(int endadd, int row) { return endadd * SD_KEY_ROWS + (SD_KEY_ROWS - 1 - row); }      // key = (u>>2)*4096 + const
 SD_HD int key_value(int key) { return key >> 12; }
 // In the deferred form the J-independent part of a row end can be "minus infinity" (a length-1 row has nothing but its
-// jump candidate); with 32-bit lanes that value times 4096 would wrap, so it is clamped before the key is formed
-// (real cells stay far above: |rel| < 2^17 by the planner's score bound).
-constexpr int SD_KEY_FLOOR = -(1 << 20);
+// jump candidate); with 32-bit lanes that value times 4096 would wrap, so it is clamped before the key is formed.
+// Real row ends stay far above: a row end scores at least J[i] + (L-1)*del + min(mismatch, 0) and Bref follows J
+// within SD_REBASE_TH/4, so rel = (row end - Bref) - (L-1)*del stays above about -2^10 + min(mismatch, 0), far from
+// the floor's -2^18.  Only length-1 rows, whose endadd is 0, reach it.  The floor is a tag-3 word like the g it
+// replaces, so that its key decodes to the lane's own row.
+constexpr int SD_KEY_FLOOR = -(1 << 20) + 3;
 SD_HD int key_floor(int z) { return z > SD_KEY_FLOOR ? z : SD_KEY_FLOOR; }
 SD_HD int key_row(int key) { return SD_KEY_ROWS - 1 - (key & (SD_KEY_ROWS - 1)); }
+
+// Column key of one lane, the operand of the sweep's per-column maximum (CREDUX / atomicMax).
+//   u       the lane's last word: U (tag 2) in the classic sweeps and in column 0 of the deferred sweep, g (tag 3)
+//           afterwards.  (u << 10) is rel*4096 + (tag << 10).
+//   kc      key_const(endadd, tie-break row) - (tag << 10) of a lane that holds a counted row end; SD_KEY_NONE for any
+//           other lane (not the last lane of its slot, or a row the --ed_thr filter dropped).  tag_off: a part of
+//           (tag << 10) that kc does not include yet
+//   counted whether the lane holds a counted row end (the forward row of the slot for Scalar32)
+//   FLOOR   deferred sweep after column 0: clamp the J-independent value first (key_floor; Scalar32 only)
+// Packed16: |rel| < 2^13 by the range proof (packed_range_ok), so a lane with kc = SD_KEY_NONE stays below every real
+// key without a select.  Scalar32 has no such bound: in the shifted domain a row never decreases, so an interior cell
+// carries about the row end's rel = (row end - Bref) - (L-1)*del, and (L-1)*|del| reaches 499,500 within the planner's
+// INF check; such a lane gets INT_MIN through a select.  A counted row end's key is its true score relative to Bref
+// (|.| < 2^19 for the same reason) times 4096 and fits 32 bits, while rel*4096 alone may not: the shift and the add
+// are done modulo 2^32.
+constexpr int SD_KEY_NONE = -(1 << 30);
+template <class P, bool FLOOR = false>
+SD_HD int lane_key(uint32_t u, int kc_lo, int kc_hi, bool counted, int tag_off = 0)
+{
+    if (P::ROWS == 2) {
+        const int klo = ((int)(u << 16) >> 6) + kc_lo - tag_off;
+        const int khi = ((int)(u & 0xffff0000u) >> 6) + kc_hi - tag_off;
+        return klo > khi ? klo : khi;
+    }
+    (void)kc_hi;
+    if (FLOOR) u = (uint32_t)key_floor((int)u);
+    return counted ? (int)((u << 10) + (uint32_t)kc_lo - (uint32_t)tag_off) : INT_MIN;
+}
 
 // --------------------------------------------------------------------------------------------
 // Geometry of one launch: how DP rows map onto lanes and where backpointers live.
@@ -422,18 +454,24 @@ SD_HD int hw_distance(const uint8_t *pat, int m, const uint8_t *text, int n, int
 //   jr[i], i=1..n : J[i] = max_r H[i-1][r][last] (jr[n].j is the final score) and its lowest row.
 //   k == 0 cells are decided here from J and the two symbols involved (main.cpp:245 tests the insertion
 //   equality at k==0 although the forward pass never takes that move, main.cpp:194).
-// Records come out last-to-first (the caller reverses, main.cpp:268).  Returns the count or -1 on overflow.
+// Records come out last-to-first (the caller reverses, main.cpp:268).  Returns the count, -1 on overflow, or
+// SD_TB_BAD_ROW when a jump names a row outside the nrows DP rows, or a filtered-out rank (a wrong column key;
+// row_off is not read then).
+constexpr int SD_TB_BAD_ROW = -2;
 template <class CodeAt>
 SD_HD int traceback_segment(int n, const JR *jr, const uint8_t *seg, const uint8_t *rows,
                             const int *row_off, int ins, int del, int mismatch, int match,
-                            CodeAt code_at, Record *out, int cap, bool writer = true, const int *rank2row = nullptr)
+                            CodeAt code_at, Record *out, int cap, bool writer = true, const int *rank2row = nullptr,
+                            int nrows = SD_KEY_ROWS)
 {
     // rank2row: with the --ed_thr pre-filter the DP rows of a segment are a re-ordered subset (main.cpp:135-149) and
-    // jr[].row holds the position in that list; rank2row maps it back to the row of the full set
+    // jr[].row holds the position in that list; rank2row maps it back to the row of the full set (-1 past its end)
     (void)del;
+    auto row_of = [&](int kr) { return (unsigned)kr >= (unsigned)nrows ? -1 : rank2row ? rank2row[kr] : kr; };
     int cnt = 0;
     int i = n - 1;
-    int r = rank2row ? rank2row[jr[n].row] : jr[n].row;
+    int r = row_of(jr[n].row);
+    if (r < 0) return SD_TB_BAD_ROW;
     int last = row_off[r + 1] - row_off[r] - 1;
     int k = last;
     int end = i;
@@ -463,7 +501,8 @@ SD_HD int traceback_segment(int n, const JR *jr, const uint8_t *seg, const uint8
         if (writer) out[cnt] = rec;
         ++cnt;
         end_score = jr[i].j;
-        r = rank2row ? rank2row[jr[i].row] : jr[i].row;
+        r = row_of(jr[i].row);
+        if (r < 0) return SD_TB_BAD_ROW;
         --i;
         last = row_off[r + 1] - row_off[r] - 1;
         k = last; end = i;

@@ -118,8 +118,9 @@ __device__ __forceinline__ void sweep_body(const SweepArgs &a)
         const int *rk = a.rank + (size_t)(first + seg_local) * (2 * a.M);
         tb_lo = rk[slot]; tb_hi = (P::ROWS == 2) ? rk[a.M + slot] : -1;
     }
-    const int kc_lo = (is_end && tb_lo >= 0) ? key_const(endadd, tb_lo) - 0x800 : -(1 << 30);
-    const int kc_hi = (is_end && tb_hi >= 0) ? key_const(endadd, tb_hi) - 0x800 : -(1 << 30);
+    const bool key_lo = is_end && tb_lo >= 0;
+    const int kc_lo = key_lo ? key_const(endadd, tb_lo) - 0x800 : SD_KEY_NONE;
+    const int kc_hi = (is_end && tb_hi >= 0) ? key_const(endadd, tb_hi) - 0x800 : SD_KEY_NONE;
     JR *jptr = a.jr + (active ? a.seg_j_off[first + seg_local] : 0);
     uint32_t *cptr = a.codes + a.cta_code_off[cta] + (size_t)tid * a.CW;
     const size_t cstride = (size_t)NT * a.CW;
@@ -192,16 +193,7 @@ __device__ __forceinline__ void sweep_body(const SweepArgs &a)
         cptr += cstride;
 
         // row ends -> (score,row) key of the segment: key = (u >> 2) * 4096 + (endadd * 4096 + 4095 - row)
-        // U = 4*rel + 2, so (half << 10) already is rel*4096 + 0x800: no masking of the low bits is needed for the
-        // forward row; lanes that hold no row end carry a very negative constant instead of a select
-        int key;
-        if (P::ROWS == 2) {
-            const int klo = ((int)(uend << 16) >> 6) + kc_lo;
-            const int khi = ((int)(uend & 0xffff0000u) >> 6) + kc_hi;
-            key = max(klo, khi);
-        } else {
-            key = ((int)uend << 10) + kc_lo;
-        }
+        const int key = lane_key<P>(uend, kc_lo, kc_hi, key_lo);
         if (FAST) {
             const int wk = __reduce_max_sync(0xffffffffu, key);
             if (lane == 0) asm volatile("st.shared.b32 [%0], %1;" ::"r"(key_wr_s + kboff), "r"(wk) : "memory");
@@ -350,8 +342,9 @@ __global__ void sweep_group_kernel(const GroupArgs a)
             const int *rk = a.rank + (size_t)seg * (2 * a.M);
             tb_lo = rk[slot]; tb_hi = (P::ROWS == 2) ? rk[a.M + slot] : -1;
         }
-        const int kc_lo = (is_end && tb_lo >= 0) ? key_const(endadd, tb_lo) - 0x800 : -(1 << 30);
-        const int kc_hi = (is_end && tb_hi >= 0) ? key_const(endadd, tb_hi) - 0x800 : -(1 << 30);
+        const bool key_lo = is_end && tb_lo >= 0;
+        const int kc_lo = key_lo ? key_const(endadd, tb_lo) - 0x800 : SD_KEY_NONE;
+        const int kc_hi = (is_end && tb_hi >= 0) ? key_const(endadd, tb_hi) - 0x800 : SD_KEY_NONE;
         JR *jptr = a.jr + (seg_ok ? a.seg_j_off[seg] : 0);
         uint32_t *cptr = a.codes + (seg_ok ? a.cta_code_off[(size_t)seg * NG + grp] : 0) + (size_t)(wseg * 32 + lane) * a.CW;
         const size_t cstride = (size_t)NT * a.CW;
@@ -386,16 +379,7 @@ __global__ void sweep_group_kernel(const GroupArgs a)
                 for (int w = 0; w < NW; ++w) cptr[w] = cw[w];
             }
             cptr += cstride;
-            // U = 4*rel + 2, so (half << 10) already is rel*4096 + 0x800: no masking of the low bits is needed for the
-            // forward row; lanes that hold no row end carry a very negative constant instead of a select
-            int key;
-            if (P::ROWS == 2) {
-                const int klo = ((int)(uend << 16) >> 6) + kc_lo;
-                const int khi = ((int)(uend & 0xffff0000u) >> 6) + kc_hi;
-                key = max(klo, khi);
-            } else {
-                key = ((int)uend << 10) + kc_lo;
-            }
+            const int key = lane_key<P>(uend, kc_lo, kc_hi, key_lo);
             const int wk = __reduce_max_sync(0xffffffffu, key);
             if (lane == 0) swk[seg_local * wps + wseg] = wk;
             uint32_t prevU = deadu;

@@ -52,6 +52,7 @@ struct TbArgs {
     int ins, del, mismatch, match;
     Record *scratch; const int64_t *seg_rec_off; int *counts;
     const int *rank2row;    // --ed_thr pre-filter: [segment][rank] -> row of the full set, or null
+    int *error;             // set to 1 when a jump names a row outside the monomer set (SD_MSG_TB_BAD_ROW)
     int invC;               // ceil(65536 / C): pos / C == (pos * invC) >> 16 for every pos < C*T (checked on the host)
 };
 
@@ -81,8 +82,14 @@ __global__ void __launch_bounds__(TB_WARPS * 32) traceback_kernel(const TbArgs a
 
     // walk state (warp-uniform)
     const int *r2r = a.rank2row ? a.rank2row + (size_t)s * (2 * g.M) : nullptr;
+    // the row of a jump comes from the sweep's column key: one outside the DP rows is reported, not used as an index
+    auto row_of = [&](int kr) { return (unsigned)kr >= (unsigned)(2 * g.M) ? -1 : r2r ? r2r[kr] : kr; };
     int i = n - 1;
-    int r = r2r ? r2r[jr[n].row] : jr[n].row;
+    int r = row_of(jr[n].row);
+    if (r < 0) {
+        if (lane == 0) { *a.error = 1; a.counts[s] = 0; }
+        return;
+    }
     int last = a.row_off[r + 1] - a.row_off[r] - 1;
     int k = last, end = i, end_score = jr[n].j, cnt = 0;
     // Window (per lane): the three words around this lane's cell, and a ring of look-ahead windows further down the
@@ -198,7 +205,12 @@ __global__ void __launch_bounds__(TB_WARPS * 32) traceback_kernel(const TbArgs a
         if (lane == 0) out[cnt] = rec;
         ++cnt;
         end_score = ji.j;
-        r = r2r ? r2r[ji.row] : ji.row;
+        r = row_of(ji.row);
+        if (r < 0) {
+            if (lane == 0) *a.error = 1;
+            cnt = 0;
+            break;
+        }
         --i;
         last = a.row_off[r + 1] - a.row_off[r] - 1;
         k = last; end = i;
@@ -456,7 +468,8 @@ struct PinnedBuf {          // page-locked host memory: the result block of a wa
 struct MetaView { void *p = nullptr; template <class U> U *as() { return reinterpret_cast<U *>(p); } };
 
 // Result block of a wave in device memory: header, per-segment counts, then the dense records.
-//   int32 flag[2] (bad symbol, exchange time-out), int32 total, int32 pad, int32 counts[nseg] (padded to 16 B), Record dense[]
+//   int32 flag[2] (bad symbol, exchange time-out), int32 total, int32 traceback row error, int32 counts[nseg] (padded to
+//   16 B), Record dense[]
 constexpr size_t OUT_HDR = 16;
 inline size_t out_counts_bytes(int nseg) { return ((size_t)nseg * 4 + 15) & ~size_t(15); }
 
@@ -801,6 +814,7 @@ public:
         t.scratch = w.d_scratch.as<Record>(); t.seg_rec_off = w.d_segrec.as<int64_t>();
         t.counts = reinterpret_cast<int *>(w.d_out.as<char>() + OUT_HDR);
         t.rank2row = w.filter_on ? w.d_r2r.as<int>() : nullptr;
+        t.error = w.d_out.as<int>() + 3;
         t.invC = (65536 + g.C - 1) / g.C;
         for (int pos = 0; pos < g.C * g.T; ++pos)
             if (((pos * t.invC) >> 16) != pos / g.C) throw PlanError{"internal: reciprocal division inexact"};
@@ -837,8 +851,9 @@ public:
     {
         SD_CUDA(cudaEventSynchronize(w.ev[5]));
         const int *hdr = w.h_out.as<int>();
-        if (hdr[0] || hdr[1]) {
+        if (hdr[0] || hdr[1] || hdr[3]) {
             if (hdr[1]) throw PlanError{"CUDA: sweep timed out waiting for a partner CTA (internal error)"};
+            if (hdr[3]) throw PlanError{SD_MSG_TB_BAD_ROW};
             throw PlanError{"segment contains a symbol outside ACGTN"};
         }
         const int64_t total = hdr[2];
@@ -907,10 +922,11 @@ public:
         WaveSlot &w = slot_[0];
         SD_CUDA(cudaMemsetAsync(w.d_out.p, 0, OUT_HDR, st_));
         enqueue_kernels(w);
-        int flag[2] = {0, 0};
-        SD_CUDA(cudaMemcpyAsync(flag, w.d_out.p, 8, cudaMemcpyDeviceToHost, st_tb_));
+        int flag[4] = {0, 0, 0, 0};
+        SD_CUDA(cudaMemcpyAsync(flag, w.d_out.p, OUT_HDR, cudaMemcpyDeviceToHost, st_tb_));
         SD_CUDA(cudaStreamSynchronize(st_tb_));
         if (flag[1]) throw PlanError{"CUDA: sweep timed out waiting for a partner CTA (internal error)"};
+        if (flag[3]) throw PlanError{SD_MSG_TB_BAD_ROW};
         if (flag[0]) throw PlanError{"segment contains a symbol outside ACGTN"};
         float ms = 0;
         SD_CUDA(cudaEventElapsedTime(&ms, w.ev[2], w.ev[3])); sweep_ms += ms;

@@ -143,8 +143,9 @@ __global__ void sweep_lat_kernel(const LatArgs a)
         tb_lo = rk[slot]; tb_hi = (P::ROWS == 2) ? rk[a.M + slot] : -1;
     }
     // key = (half << 10) + const: the row-end word is U (tag 2: 0x800 too much) in column 0, g (tag 3: 0xC00) afterwards
-    const int kc_lo = (is_end && tb_lo >= 0) ? key_const(endadd, tb_lo) : -(1 << 30);
-    const int kc_hi = (is_end && tb_hi >= 0) ? key_const(endadd, tb_hi) : -(1 << 30);
+    const bool key_lo = is_end && tb_lo >= 0;
+    const int kc_lo = key_lo ? key_const(endadd, tb_lo) : SD_KEY_NONE;
+    const int kc_hi = (is_end && tb_hi >= 0) ? key_const(endadd, tb_hi) : SD_KEY_NONE;
     const int kc3_lo = kc_lo - 0xC00, kc3_hi = kc_hi - 0xC00;
     JR *jptr = a.jr + a.seg_j_off[seg];
     uint32_t *cptr = a.codes + a.cta_code_off[(size_t)seg * NG + grp] + (size_t)tid * a.CW;
@@ -255,10 +256,7 @@ __global__ void sweep_lat_kernel(const LatArgs a)
         uint32_t ufirst;
         const uint32_t uend = lane_pass2_pre<P, C>(X, carry, cw, tr, pw, deadu, kill_last, &ufirst);
         store_codes();
-        int key;
-        if (P::ROWS == 2) key = max(((int)(uend << 16) >> 6) + kc_lo - 0x800, ((int)(uend & 0xffff0000u) >> 6) + kc_hi - 0x800);
-        else key = ((int)uend << 10) + kc_lo - 0x800;
-        publish(0u, 1, __reduce_max_sync(0xffffffffu, key));
+        publish(0u, 1, __reduce_max_sync(0xffffffffu, lane_key<P>(uend, kc_lo, kc_hi, key_lo, 0x800)));
         uint32_t prevU = deadu;
         if (T > 1) { prevU = __shfl_up_sync(0xffffffffu, uend, 1); if (t == 0) prevU = deadu; }
         X[0] = lane_pre_first<P>(prevU, pw[0], ufirst, deadu, kill_first, C == 1 && kill_last);
@@ -296,10 +294,7 @@ __global__ void sweep_lat_kernel(const LatArgs a)
         load_p(pn);                                       // flies during the chain
         const uint32_t g = lat_chain<P, C>(X, carry, trr);
         tick(1);
-        int key;
-        if (P::ROWS == 2) key = max(((int)(g << 16) >> 6) + kc3_lo, ((int)(g & 0xffff0000u) >> 6) + kc3_hi);
-        else key = (key_floor((int)g) << 10) + kc3_lo;
-        publish(boff, i + 1, __reduce_max_sync(0xffffffffu, key));
+        publish(boff, i + 1, __reduce_max_sync(0xffffffffu, lane_key<P, true>(g, kc3_lo, kc3_hi, key_lo)));
         tick(2);
 
         // J[i] from the key of column i-1, published one column ago

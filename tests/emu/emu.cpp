@@ -7,6 +7,7 @@
 #include <algorithm>
 #include <climits>
 #include <cstring>
+#include <type_traits>
 
 #include "common.h"
 #include "identity_core.cuh"
@@ -17,6 +18,7 @@ namespace {
 
 bool &bad_symbol() { static thread_local bool f = false; return f; }
 bool &window_violation() { static thread_local bool f = false; return f; }
+bool &key_violation() { static thread_local bool f = false; return f; }
 
 template <class P, int C, int T>
 void emu_cta(const Plan &p, const Batch &b, int seg_first, int nseg_cta, int nmax,
@@ -33,7 +35,8 @@ void emu_cta(const Plan &p, const Batch &b, int seg_first, int nseg_cta, int nma
     std::vector<uint32_t> Xall((size_t)NT * C, deadu), PWall((size_t)NT * C, 0u);
     std::vector<uint32_t> E(NT), carry(NT);
     std::vector<int> bref(NS, p.sc.ins), jump0(NS, 0);
-    std::vector<int> key(NS, INT_MIN);
+    // key: the column key formed with a select over the counted row ends; dkey: the same with the kernels' arithmetic
+    std::vector<int> key(NS, INT_MIN), dkey(NS, INT_MIN);
     uint32_t (*X)[C] = reinterpret_cast<uint32_t (*)[C]>(Xall.data());
     uint32_t (*PW)[C] = reinterpret_cast<uint32_t (*)[C]>(PWall.data());
     uint32_t cw[8];
@@ -89,6 +92,7 @@ void emu_cta(const Plan &p, const Batch &b, int seg_first, int nseg_cta, int nma
             carry[tid] = win;
         }
         std::fill(key.begin(), key.end(), INT_MIN);
+        std::fill(dkey.begin(), dkey.end(), INT_MIN);
         for (int tid = 0; tid < NT; ++tid) {
             const LaneId l = lane_id(tid);
             load_profile(tid, l, i + 1);                      // profile of the next column (0-padded past the end)
@@ -96,17 +100,27 @@ void emu_cta(const Plan &p, const Batch &b, int seg_first, int nseg_cta, int nma
                                              l.t == T - 1 && p.slot_len[l.slot] == 1, &ufirst[tid]);
             if (l.active && i < l.n)
                 for (int w = 0; w < g.CW; ++w) codes[tid / NTC][((size_t)i * NTC + tid % NTC) * g.CW + w] = cw[w];
-            if (l.active && l.t == T - 1) {
-                const uint32_t u = uend[tid];
-                const int R = 2 * g.M;
-                int row_lo = l.slot, row_hi = g.M + l.slot;                  // tie-break index of the two rows of the slot
-                if (rank) { row_lo = rank[l.seg_local * R + row_lo]; row_hi = (P::ROWS == 2) ? rank[l.seg_local * R + row_hi] : -1; }
+            const bool is_end = l.active && l.t == T - 1;
+            const uint32_t u = uend[tid];
+            const int R = 2 * g.M;
+            int row_lo = l.slot, row_hi = g.M + l.slot;                      // tie-break index of the two rows of the slot
+            if (rank && l.active) { row_lo = rank[l.seg_local * R + row_lo]; row_hi = (P::ROWS == 2) ? rank[l.seg_local * R + row_hi] : -1; }
+            if (is_end) {
                 int k0 = INT_MIN;
                 if (row_lo >= 0) k0 = make_key(P::lo(u), p.slot_endadd[l.slot], row_lo);
                 if (P::ROWS == 2 && row_hi >= 0) k0 = std::max(k0, make_key(P::hi(u), p.slot_endadd[l.slot], row_hi));
                 key[l.seg_local] = std::max(key[l.seg_local], k0);
             }
+            // the kernels' key of every lane (an idle lane counts towards the segment of its warp, as in the warp reduction)
+            if (l.seg_local < nseg_cta) {
+                const int endadd = p.slot_endadd[l.slot];
+                const int kc_lo = (is_end && row_lo >= 0) ? key_const(endadd, row_lo) - 0x800 : SD_KEY_NONE;
+                const int kc_hi = (is_end && row_hi >= 0) ? key_const(endadd, row_hi) - 0x800 : SD_KEY_NONE;
+                dkey[l.seg_local] = std::max(dkey[l.seg_local], lane_key<P>(u, kc_lo, kc_hi, is_end && row_lo >= 0));
+            }
         }
+        for (int s = 0; s < nseg_cta; ++s)
+            if (i < b.len(seg_first + s) && dkey[s] != key[s]) key_violation() = true;
         for (int tid = 0; tid < NT; ++tid) {
             const LaneId l = lane_id(tid);
             const uint32_t prevU = (l.t == 0) ? deadu : uend[tid - 1];
@@ -192,7 +206,15 @@ void emu_cta_lat(const Plan &p, const Batch &b, int seg_first, int nseg_cta, int
         E[tid] = lane_post<P, C>(X[tid], PW[tid], P::splat(0 + 1), deadu, tr);
     }
     for (int tid = 0; tid < NT; ++tid) carry[tid] = (lane_id(tid).t == 0) ? deadu : P::max2(carry[tid - 1], E[tid - 1]);
+    // the kernel's key of a lane (sweep_lat_kernel: kc_lo / kc3_lo); tag_off 0x800 in column 0, 0xC00 afterwards
+    auto device_key = [&](const LaneId &l, uint32_t u, int tag_off, auto floor) {
+        const bool is_end = l.active && l.t == T - 1;
+        const int kc_lo = (is_end && tie_lo(l) >= 0) ? key_const(p.slot_endadd[l.slot], tie_lo(l)) : SD_KEY_NONE;
+        const int kc_hi = (is_end && tie_hi(l) >= 0) ? key_const(p.slot_endadd[l.slot], tie_hi(l)) : SD_KEY_NONE;
+        return lane_key<P, decltype(floor)::value>(u, kc_lo, kc_hi, is_end && tie_lo(l) >= 0, tag_off);
+    };
     int kpub = INT_MIN;                                  // key published for the column just swept
+    int dkey = INT_MIN;
     for (int tid = 0; tid < NT; ++tid) {
         const LaneId l = lane_id(tid);
         load_profile(tid, l, 1);
@@ -203,7 +225,9 @@ void emu_cta_lat(const Plan &p, const Batch &b, int seg_first, int nseg_cta, int
             if (tie_lo(l) >= 0) kpub = std::max(kpub, make_key(P::lo(uend[tid]), p.slot_endadd[l.slot], tie_lo(l)));
             if (tie_hi(l) >= 0) kpub = std::max(kpub, make_key(P::hi(uend[tid]), p.slot_endadd[l.slot], tie_hi(l)));
         }
+        dkey = std::max(dkey, device_key(l, uend[tid], 0x800, std::false_type()));
     }
+    if (dkey != kpub) key_violation() = true;
     for (int tid = 0; tid < NT; ++tid) {
         const LaneId l = lane_id(tid);
         const uint32_t prevU = (l.t == 0) ? deadu : uend[tid - 1];
@@ -229,6 +253,7 @@ void emu_cta_lat(const Plan &p, const Batch &b, int seg_first, int nseg_cta, int
             carry[tid] = win;
         }
         int knew = INT_MIN;
+        dkey = INT_MIN;
         for (int tid = 0; tid < NT; ++tid) {
             const LaneId l = lane_id(tid);
             gout[tid] = lat_chain<P, C>(X[tid], carry[tid], tr);
@@ -236,7 +261,9 @@ void emu_cta_lat(const Plan &p, const Batch &b, int seg_first, int nseg_cta, int
                 if (tie_lo(l) >= 0) knew = std::max(knew, make_key(P::ROWS == 2 ? P::lo(gout[tid]) : key_floor(P::lo(gout[tid])), p.slot_endadd[l.slot], tie_lo(l)));
                 if (tie_hi(l) >= 0) knew = std::max(knew, make_key(P::hi(gout[tid]), p.slot_endadd[l.slot], tie_hi(l)));
             }
+            dkey = std::max(dkey, device_key(l, gout[tid], 0xC00, std::true_type()));
         }
+        if (dkey != knew) key_violation() = true;
         // c. the key of column i-1 arrives: J[i]
         consume(i);
         kpub = knew;
@@ -361,6 +388,7 @@ public:
         }
         overflowed_ = g.packed && EmuFlags::overflow();
         if (window_violation()) { window_violation() = false; throw PlanError{"emulator: windowed deletion carry differs from the full prefix maximum (scan_window too small)"}; }
+        if (key_violation()) { key_violation() = false; throw PlanError{"emulator: the kernels' column key differs from the select-based key (key_violation)"}; }
         if (bad_symbol()) throw PlanError{"segment contains a symbol outside ACGTN"};
         // the traceback compares segment and row symbols: bring the rows to the same (ASCII) alphabet
         rows_ascii_.resize(ms_.rows.size());
@@ -369,6 +397,9 @@ public:
         // traceback
         recs_.assign((size_t)lay_.seg_rec_off.back(), Record{});
         cnt_.assign(nseg, 0);
+        // SD_EMU_BAD_JUMP_ROW=1 (tests): the last jump of the first segment names row 4095, as a wrong column key would
+        if (getenv("SD_EMU_BAD_JUMP_ROW") && atoi(getenv("SD_EMU_BAD_JUMP_ROW")) && nseg > 0)
+            jr_[(size_t)lay_.seg_j_off[0] + b.len(s0_)].row = SD_KEY_ROWS - 1;
         for (int s = 0; s < nseg; ++s) {
             const int n = b.len(s0_ + s);
             if (n == 0) continue;
@@ -382,7 +413,7 @@ public:
                                         b.text + b.off[s0_ + s], rows_ascii_.data(), ms_.row_off.data(),
                                         plan_.sc.ins, plan_.sc.del, plan_.sc.mismatch, plan_.sc.match, code_at,
                                         recs_.data() + lay_.seg_rec_off[s], n, true,
-                                        r2r_.empty() ? nullptr : r2r_.data() + (size_t)s * ms_.nrows());
+                                        r2r_.empty() ? nullptr : r2r_.data() + (size_t)s * ms_.nrows(), ms_.nrows());
         }
     }
     void fetch(BatchResult &out) override
@@ -390,6 +421,7 @@ public:
         if (overflowed_) throw PlanError{"emulator: 16-bit overflow in the packed sweep (range proof violated)"};
         const int nseg = s1_ - s0_;
         for (int s = 0; s < nseg; ++s) {
+            if (cnt_[s] == SD_TB_BAD_ROW) throw PlanError{SD_MSG_TB_BAD_ROW};
             if (cnt_[s] < 0) throw PlanError{"emulator: traceback record overflow"};
             const Record *r = recs_.data() + lay_.seg_rec_off[s];
             for (int x = cnt_[s] - 1; x >= 0; --x) out.recs.push_back(r[x]);
