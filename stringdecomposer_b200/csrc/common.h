@@ -62,6 +62,14 @@ SD_HD int ascii_code(unsigned c)
 {
     return c == 'A' ? 0 : c == 'C' ? 1 : c == 'G' ? 2 : c == 'T' ? 3 : c == 'N' ? 4 : 255;
 }
+// Symbol code of a segment byte for the sweeps: a byte outside ACGTN sets *bad (the host then refuses the wave) and
+// reads as 0, so the sweep stays in range until then
+SD_HD int symbol_code(unsigned c, int *bad)
+{
+    int code = ascii_code(c);
+    if (code > 4) { *bad = 1; code = 0; }
+    return code;
+}
 
 struct BatchResult {
     std::vector<Record> recs;            // per segment in read order (already reversed), positions segment-relative

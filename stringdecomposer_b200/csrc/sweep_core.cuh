@@ -146,6 +146,19 @@ SD_HD void lane_pre(uint32_t (&X)[C], uint32_t prevU, const uint32_t *pw, uint32
     }
 }
 
+// Pass 1a of column 0, where every cell of the previous column is dead and the base is B[0] = ins (row-0 rule,
+// main.cpp:180).  A row's k==0 cell is s(0,0) itself (main.cpp:173-177), one `del` more than the generic jump
+// candidate, so the profile word of the slot's first cell (the last cell of a length-1 row) gets 4*del added first.
+// del is taken by reference so that a kernel reads its parameter where it uses it: passed by value, the load moves
+// ahead of the two branches and the kernels' machine code changes.
+template <class P, int C>
+SD_HD void lane_pre_col0(uint32_t (&X)[C], uint32_t *pw, const int &del, int L, uint32_t deadu, bool kill_first, bool kill_last)
+{
+    if (kill_first && L > 1) pw[0] = P::add(pw[0], P::splat(4 * del));
+    if (kill_last) pw[C - 1] = P::add(pw[C - 1], P::splat(4 * del));
+    lane_pre<P, C>(X, deadu, pw, deadu, kill_first, kill_last);
+}
+
 // Pass 1b ("post"): add the jump candidate 4*(B[i]-Bref) + 4*s'' (tag 0) once J[i] is known.
 // jump0p1 = splat(4*(B[i]-Bref) + 1) (the +1 undoes the -1 folded into the profile words).
 // Returns the lane maximum in tag-2 form: what the lane hands to the lanes on its right (deletion chain).
@@ -349,6 +362,29 @@ SD_HD int lane_key(uint32_t u, int kc_lo, int kc_hi, bool counted, int tag_off =
     (void)kc_hi;
     if (FLOOR) u = (uint32_t)key_floor((int)u);
     return counted ? (int)((u << 10) + (uint32_t)kc_lo - (uint32_t)tag_off) : INT_MIN;
+}
+
+// lane_key's constants for one lane of a slot.  is_end: the lane is the active last lane of its slot.  Ties between
+// rows break on the row itself, or with the --ed_thr pre-filter on its position in the segment's filtered list
+// (main.cpp:141-147): rank is the [segment][row] -> position table (-1 = filtered out) or null, read only for an active
+// lane, at segment first + seg (a classic sweep CTA holds segments first, first+1, ...).  kc_off is added to the
+// constant of every counted row (the part of -(tag << 10) the caller folds in).  The segment comes in two parts and M
+// by reference for the reason given at lane_pre_col0: the kernels then form the rank address and read M inside the
+// branches that use them.
+struct SlotKey { int kc_lo, kc_hi; bool counted; };
+template <class P>
+SD_HD SlotKey slot_key(bool active, bool is_end, int endadd, int slot, const int &M, const int *rank, int first, int seg, int kc_off)
+{
+    int tb_lo = slot, tb_hi = M + slot;
+    if (rank && active) {
+        const int *rk = rank + (size_t)(first + seg) * (2 * M);
+        tb_lo = rk[slot]; tb_hi = (P::ROWS == 2) ? rk[M + slot] : -1;
+    }
+    SlotKey k;
+    k.counted = is_end && tb_lo >= 0;
+    k.kc_lo = k.counted ? key_const(endadd, tb_lo) + kc_off : SD_KEY_NONE;
+    k.kc_hi = (is_end && tb_hi >= 0) ? key_const(endadd, tb_hi) + kc_off : SD_KEY_NONE;
+    return k;
 }
 
 // --------------------------------------------------------------------------------------------

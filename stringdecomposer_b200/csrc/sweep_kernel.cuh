@@ -55,6 +55,40 @@ __device__ __forceinline__ uint32_t slot_scan_window(uint32_t E, int t, uint32_t
     return pv;
 }
 
+// Profile words of one lane for one column: (C+3)/4 uint4 loads from the lane's row of the symbol (the words past C are
+// padding).
+template <int C>
+__device__ __forceinline__ void load_profile_row(uint32_t (&pw)[(C + 3) / 4 * 4], const uint4 *row)
+{
+#pragma unroll
+    for (int q = 0; q < (C + 3) / 4; ++q) {
+        const uint4 v = row[q];
+        pw[4 * q] = v.x; pw[4 * q + 1] = v.y; pw[4 * q + 2] = v.z; pw[4 * q + 3] = v.w;
+    }
+}
+
+// One lane's backpointer words of one column: a single vector store where the word count allows it.
+template <int NW>
+__device__ __forceinline__ void store_code_words(uint32_t *cptr, const uint32_t (&cw)[NW])
+{
+    if (NW == 2) *reinterpret_cast<uint2 *>(cptr) = make_uint2(cw[0], cw[1]);
+    else if (NW == 4) *reinterpret_cast<uint4 *>(cptr) = make_uint4(cw[0], cw[1], cw[2], cw[3]);
+    else {
+#pragma unroll
+        for (int w = 0; w < NW; ++w) cptr[w] = cw[w];
+    }
+}
+
+// First cell of the lane for the next column (lane_pre_first): it needs the left lane's row-end value.
+template <class P, int C, int T>
+__device__ __forceinline__ uint32_t next_first_cell(uint32_t uend, uint32_t pn0, uint32_t ufirst, uint32_t deadu, int t,
+                                                    bool kill_first, bool kill_last)
+{
+    uint32_t prevU = deadu;
+    if (T > 1) { prevU = __shfl_up_sync(0xffffffffu, uend, 1); if (t == 0) prevU = deadu; }
+    return lane_pre_first<P>(prevU, pn0, ufirst, deadu, kill_first, C == 1 && kill_last);
+}
+
 // FAST: every warp serves exactly one segment and a segment has <= 4 warps: the per-column (score,row) key is
 // reduced with CREDUX inside the warp and exchanged through one aligned int4 row of shared memory.
 // MULTI (with FAST): several segments share the CTA and its profile table but synchronise separately (named barriers).
@@ -96,11 +130,7 @@ __device__ __forceinline__ void sweep_body(const SweepArgs &a)
             n = (int)(a.seg_off[first + s + 1] - o);
             src = a.bases + o;
         }
-        for (int x = tid; x < a.seg_stride; x += NT) {
-            int code = (x < n) ? ascii_code(src[x]) : 0;
-            if (code > 4) { *a.bad_symbol = 1; code = 0; }
-            schar[s * a.seg_stride + x] = (uint8_t)code;
-        }
+        for (int x = tid; x < a.seg_stride; x += NT) schar[s * a.seg_stride + x] = (uint8_t)((x < n) ? symbol_code(src[x], a.bad_symbol) : 0);
     }
     for (int x = tid; x < 3 * kstride; x += NT) skey[x] = INT_MIN;
     __syncthreads();
@@ -112,26 +142,14 @@ __device__ __forceinline__ void sweep_body(const SweepArgs &a)
     const bool kill_first = (t == 0), kill_last = (t == T - 1 && L == 1);
     const bool j_writer = active && slot == 0 && t == 0;
     const bool is_end = active && t == T - 1;
-    // tie-break index of the slot's rows: the row itself, or its position in the segment's filtered list (main.cpp:141-147)
-    int tb_lo = slot, tb_hi = a.M + slot;
-    if (a.rank && active) {
-        const int *rk = a.rank + (size_t)(first + seg_local) * (2 * a.M);
-        tb_lo = rk[slot]; tb_hi = (P::ROWS == 2) ? rk[a.M + slot] : -1;
-    }
-    const bool key_lo = is_end && tb_lo >= 0;
-    const int kc_lo = key_lo ? key_const(endadd, tb_lo) - 0x800 : SD_KEY_NONE;
-    const int kc_hi = (is_end && tb_hi >= 0) ? key_const(endadd, tb_hi) - 0x800 : SD_KEY_NONE;
+    const SlotKey sk = slot_key<P>(active, is_end, endadd, slot, a.M, a.rank, first, seg_local, -0x800);
     JR *jptr = a.jr + (active ? a.seg_j_off[first + seg_local] : 0);
     uint32_t *cptr = a.codes + a.cta_code_off[cta] + (size_t)tid * a.CW;
     const size_t cstride = (size_t)NT * a.CW;
     const uint8_t *cp = schar + seg_local * a.seg_stride;               // symbol of the column being prepared
     // STREAM: the segment's text in global memory; columns past its end read as symbol 0, like the 0-padded buffer
     const uint8_t *src = a.bases + (active ? a.seg_off[first + seg_local] : 0);
-    auto symbol = [&](int i) {
-        int code = (i < n_seg) ? ascii_code(__ldg(src + i)) : 0;
-        if (code > 4) { *a.bad_symbol = 1; code = 0; }
-        return code;
-    };
+    auto symbol = [&](int i) { return (i < n_seg) ? symbol_code(__ldg(src + i), a.bad_symbol) : 0; };
     const uint4 *myprof = sprof + (size_t)(slot * T + t) * a.qp;
     const int sym_stride = a.nsl * a.qp;
     // FAST: segment s of the CTA owns int4 row s of each key buffer, its warps write one int each.  Raw shared-space
@@ -143,27 +161,15 @@ __device__ __forceinline__ void sweep_body(const SweepArgs &a)
     const uint32_t kbytes = 4u * (uint32_t)kstride;
     const int bar_id = 1 + wseg, bar_threads = a.wps * 32;
 
-    constexpr int CQ = (C + 3) / 4;                     // uint4 profile loads per lane (the tail words are padding)
-    uint32_t X[C], pw[CQ * 4];
+    uint32_t X[C], pw[(C + 3) / 4 * 4];
 #pragma unroll
     for (int kk = 0; kk < C; ++kk) X[kk] = deadu;
-    auto load_profile = [&](int sym) {
-        const uint4 *pp = myprof + sym * sym_stride;
-#pragma unroll
-        for (int q = 0; q < CQ; ++q) {
-            const uint4 v = pp[q];
-            pw[4 * q] = v.x; pw[4 * q + 1] = v.y; pw[4 * q + 2] = v.z; pw[4 * q + 3] = v.w;
-        }
-    };
+    auto load_profile = [&](int sym) { load_profile_row<C>(pw, myprof + sym * sym_stride); };
 
-    // column 0: everything dead, base B[0] = ins (row-0 rule, main.cpp:180); the k==0 cell is s(0,0) itself
-    // (main.cpp:173-177), i.e. one `del` more than the generic jump candidate
     int sym_next = 0;
     if (STREAM) { load_profile(symbol(0)); sym_next = symbol(1); }
     else load_profile(*cp++);
-    if (t == 0 && L > 1) pw[0] = P::add(pw[0], P::splat(4 * a.del));
-    if (t == T - 1 && L == 1) pw[C - 1] = P::add(pw[C - 1], P::splat(4 * a.del));
-    lane_pre<P, C>(X, deadu, pw, deadu, kill_first, kill_last);
+    lane_pre_col0<P, C>(X, pw, a.del, L, deadu, kill_first, kill_last);
     int jbase = a.ins;            // Bref + i*ins: J[i+1] = vmax + jbase
     int jump0 = 0;                // 4*(B[i] - Bref)
     uint32_t kboff = 0;           // byte offset of the key buffer in use (FAST: 2 buffers alternate; else 3 rotate)
@@ -182,18 +188,11 @@ __device__ __forceinline__ void sweep_body(const SweepArgs &a)
 
         // one segment per CTA (FAST without MULTI): every column is live; else a shorter segment idles past its end
         const bool live = active && ((FAST && !MULTI) || i < n_seg);
-        if (live) {
-            if (NW == 2) *reinterpret_cast<uint2 *>(cptr) = make_uint2(cw[0], cw[1]);
-            else if (NW == 4) *reinterpret_cast<uint4 *>(cptr) = make_uint4(cw[0], cw[1], cw[2], cw[3]);
-            else {
-#pragma unroll
-                for (int w = 0; w < NW; ++w) cptr[w] = cw[w];
-            }
-        }
+        if (live) store_code_words(cptr, cw);
         cptr += cstride;
 
         // row ends -> (score,row) key of the segment: key = (u >> 2) * 4096 + (endadd * 4096 + 4095 - row)
-        const int key = lane_key<P>(uend, kc_lo, kc_hi, key_lo);
+        const int key = lane_key<P>(uend, sk.kc_lo, sk.kc_hi, sk.counted);
         if (FAST) {
             const int wk = __reduce_max_sync(0xffffffffu, key);
             if (lane == 0) asm volatile("st.shared.b32 [%0], %1;" ::"r"(key_wr_s + kboff), "r"(wk) : "memory");
@@ -204,10 +203,7 @@ __device__ __forceinline__ void sweep_body(const SweepArgs &a)
             if (tid < NS) asm volatile("st.shared.b32 [%0], %1;" ::"r"(skey_s + kclr + 4u * tid), "r"(INT_MIN) : "memory");
             if (is_end) atomicMax(reinterpret_cast<int *>(reinterpret_cast<char *>(skey) + kboff) + seg_local, key);
         }
-        // first cell of the lane for the next column: needs the left lane's row-end value
-        uint32_t prevU = deadu;
-        if (T > 1) { prevU = __shfl_up_sync(0xffffffffu, uend, 1); if (t == 0) prevU = deadu; }
-        X[0] = lane_pre_first<P>(prevU, pw[0], ufirst, deadu, kill_first, C == 1 && kill_last);
+        X[0] = next_first_cell<P, C, T>(uend, pw[0], ufirst, deadu, t, kill_first, kill_last);
         // (ptxas schedules these J-independent max-plus ops behind the barrier, where they cover the latency of the
         // key load that follows it)
 
@@ -312,16 +308,8 @@ __global__ void sweep_group_kernel(const GroupArgs a)
     unsigned gcol = 0;                                   // columns this CTA group has exchanged so far
     __syncthreads();
 
-    constexpr int CQ = (C + 3) / 4;
-    uint32_t X[C], pw[CQ * 4];
-    auto load_profile = [&](int sym) {
-        const uint4 *pp = myprof + sym * sym_stride;
-#pragma unroll
-        for (int q = 0; q < CQ; ++q) {
-            const uint4 v = pp[q];
-            pw[4 * q] = v.x; pw[4 * q + 1] = v.y; pw[4 * q + 2] = v.z; pw[4 * q + 3] = v.w;
-        }
-    };
+    uint32_t X[C], pw[(C + 3) / 4 * 4];
+    auto load_profile = [&](int sym) { load_profile_row<C>(pw, myprof + sym * sym_stride); };
     const int nblocks = (a.nseg + NS - 1) / NS;
     for (int blk = gslot; blk < nblocks; blk += a.ngslots) {
         // the NS segments of the block advance in lockstep; a shorter (or missing) one idles past its end
@@ -337,30 +325,17 @@ __global__ void sweep_group_kernel(const GroupArgs a)
         const bool active = slot_ok && seg_ok;
         const bool is_end = active && t == T - 1;
         const bool j_writer = seg_ok && grp == 0 && wseg == 0 && lane == 0;
-        int tb_lo = slot, tb_hi = a.M + slot;
-        if (a.rank && active) {
-            const int *rk = a.rank + (size_t)seg * (2 * a.M);
-            tb_lo = rk[slot]; tb_hi = (P::ROWS == 2) ? rk[a.M + slot] : -1;
-        }
-        const bool key_lo = is_end && tb_lo >= 0;
-        const int kc_lo = key_lo ? key_const(endadd, tb_lo) - 0x800 : SD_KEY_NONE;
-        const int kc_hi = (is_end && tb_hi >= 0) ? key_const(endadd, tb_hi) - 0x800 : SD_KEY_NONE;
+        const SlotKey sk = slot_key<P>(active, is_end, endadd, slot, a.M, a.rank, seg, 0, -0x800);
         JR *jptr = a.jr + (seg_ok ? a.seg_j_off[seg] : 0);
         uint32_t *cptr = a.codes + (seg_ok ? a.cta_code_off[(size_t)seg * NG + grp] : 0) + (size_t)(wseg * 32 + lane) * a.CW;
         const size_t cstride = (size_t)NT * a.CW;
         // symbols are streamed from global memory (one byte per column, the same for all lanes of the segment)
         const uint8_t *src = a.bases + o;
-        auto symbol = [&](int i) {
-            int code = (i < n) ? ascii_code(__ldg(src + i)) : 0;
-            if (code > 4) { *a.bad_symbol = 1; code = 0; }
-            return code;
-        };
+        auto symbol = [&](int i) { return (i < n) ? symbol_code(__ldg(src + i), a.bad_symbol) : 0; };
 #pragma unroll
         for (int kk = 0; kk < C; ++kk) X[kk] = deadu;
         load_profile(symbol(0));
-        if (t == 0 && L > 1) pw[0] = P::add(pw[0], P::splat(4 * a.del));
-        if (t == T - 1 && L == 1) pw[C - 1] = P::add(pw[C - 1], P::splat(4 * a.del));
-        lane_pre<P, C>(X, deadu, pw, deadu, kill_first, kill_last);
+        lane_pre_col0<P, C>(X, pw, a.del, L, deadu, kill_first, kill_last);
         int jbase = a.ins, jump0 = 0;
         int sym_next = symbol(1);
 #pragma unroll 1
@@ -379,12 +354,10 @@ __global__ void sweep_group_kernel(const GroupArgs a)
                 for (int w = 0; w < NW; ++w) cptr[w] = cw[w];
             }
             cptr += cstride;
-            const int key = lane_key<P>(uend, kc_lo, kc_hi, key_lo);
+            const int key = lane_key<P>(uend, sk.kc_lo, sk.kc_hi, sk.counted);
             const int wk = __reduce_max_sync(0xffffffffu, key);
             if (lane == 0) swk[seg_local * wps + wseg] = wk;
-            uint32_t prevU = deadu;
-            if (T > 1) { prevU = __shfl_up_sync(0xffffffffu, uend, 1); if (t == 0) prevU = deadu; }
-            X[0] = lane_pre_first<P>(prevU, pw[0], ufirst, deadu, kill_first, C == 1 && kill_last);
+            X[0] = next_first_cell<P, C, T>(uend, pw[0], ufirst, deadu, t, kill_first, kill_last);
             __syncthreads();
             // Column exchange between the NG CTAs of the block (see the comment above the kernel).  Two buffers
             // suffice: a CTA can only be one column ahead of the slowest reader, because it needs everybody's key of
@@ -439,21 +412,23 @@ __global__ void sweep_group_kernel(const GroupArgs a)
     }
 }
 
-// lookup tables of the instantiations, one translation unit per (policy, FAST, MULTI, STREAM) so that they build in parallel
-const void *sweep_lookup_p16_f1_m0(int C, int T, int NT);
-const void *sweep_lookup_p16_f1_m1(int C, int T, int NT);
-const void *sweep_lookup_p16_f0_m0(int C, int T, int NT);
-const void *sweep_lookup_s32_f1_m0(int C, int T, int NT);
-const void *sweep_lookup_s32_f1_m1(int C, int T, int NT);
-const void *sweep_lookup_s32_f0_m0(int C, int T, int NT);
-const void *sweep_lookup_p16_f1_m0_st(int C, int T, int NT);
-const void *sweep_lookup_p16_f1_m1_st(int C, int T, int NT);
-const void *sweep_lookup_p16_f0_m0_st(int C, int T, int NT);
-const void *sweep_lookup_s32_f1_m0_st(int C, int T, int NT);
-const void *sweep_lookup_s32_f1_m1_st(int C, int T, int NT);
-const void *sweep_lookup_s32_f0_m0_st(int C, int T, int NT);
-const void *sweep_group_lookup_p16(int C, int T);
-const void *sweep_group_lookup_s32(int C, int T);
+// Lookup tables of the instantiations, one translation unit per (policy, FAST, MULTI, STREAM) so that they build in
+// parallel: the kernel compiled for the geometry, or null.  sweep_kernels.cu: sweep_kernel_for picks the table.
+using SweepLookup = const void *(*)(const Geometry &g);
+const void *sweep_lookup_p16_f1_m0(const Geometry &g);
+const void *sweep_lookup_p16_f1_m1(const Geometry &g);
+const void *sweep_lookup_p16_f0_m0(const Geometry &g);
+const void *sweep_lookup_s32_f1_m0(const Geometry &g);
+const void *sweep_lookup_s32_f1_m1(const Geometry &g);
+const void *sweep_lookup_s32_f0_m0(const Geometry &g);
+const void *sweep_lookup_p16_f1_m0_st(const Geometry &g);
+const void *sweep_lookup_p16_f1_m1_st(const Geometry &g);
+const void *sweep_lookup_p16_f0_m0_st(const Geometry &g);
+const void *sweep_lookup_s32_f1_m0_st(const Geometry &g);
+const void *sweep_lookup_s32_f1_m1_st(const Geometry &g);
+const void *sweep_lookup_s32_f0_m0_st(const Geometry &g);
+const void *sweep_group_lookup_p16(const Geometry &g);
+const void *sweep_group_lookup_s32(const Geometry &g);
 
 // the register-capped twin is instantiated only where it is used: several segments per CTA (LL) and C <= 24
 template <class POLICY, int CC, int TT, bool FAST, bool LL, bool ST> static const void *sweep_pick(bool cap80)
@@ -477,10 +452,11 @@ template <class POLICY, int CC, int TT, bool FAST, bool LL, bool ST> static cons
         }                                                                                                             \
         return nullptr;                                                                                               \
     }                                                                                                                 \
-    const void *NAME(int C, int T, int NT)                                                                            \
+    const void *NAME(const Geometry &g)                                                                               \
     {                                                                                                                 \
-        const bool cap80 = NT <= 768;                                                                                 \
-        switch (C) {                                                                                                  \
+        const int T = g.T;                                                                                            \
+        const bool cap80 = g.NT <= 768;                                                                               \
+        switch (g.C) {                                                                                                \
         case 8: return NAME##_t<8>(T, cap80); case 12: return NAME##_t<12>(T, cap80); case 16: return NAME##_t<16>(T, cap80);   \
         case 19: return NAME##_t<19>(T, cap80); case 20: return NAME##_t<20>(T, cap80); case 24: return NAME##_t<24>(T, cap80); \
         case 32: return NAME##_t<32>(T, cap80);                                                                       \
@@ -503,9 +479,10 @@ template <class POLICY, int CC, int TT, bool FAST, bool LL, bool ST> static cons
         }                                                                                                             \
         return nullptr;                                                                                               \
     }                                                                                                                 \
-    const void *NAME(int C, int T)                                                                                    \
+    const void *NAME(const Geometry &g)                                                                               \
     {                                                                                                                 \
-        switch (C) {                                                                                                  \
+        const int T = g.T;                                                                                            \
+        switch (g.C) {                                                                                                \
         case 8: return NAME##_t<8>(T); case 12: return NAME##_t<12>(T); case 16: return NAME##_t<16>(T);              \
         case 19: return NAME##_t<19>(T); case 20: return NAME##_t<20>(T); case 24: return NAME##_t<24>(T);              \
         case 32: return NAME##_t<32>(T);            \

@@ -393,14 +393,25 @@ template <int MODE> __global__ void int_peak_kernel(unsigned *out, unsigned seed
 }
 
 // ---------------------------------------------------------------------------------------------
-static const void *kern(int packed, int C, int T, int NT, bool fast, bool multi, bool stream)
+// The sweep kernel compiled for a geometry, or null.  fast, multi: the classic sweep's FAST and MULTI variants
+// (sweep_kernel.cuh); timing: the instrumented twin of the deferred-jump sweep (SD_LAT_TIMING; packed, staged only).
+static const void *sweep_kernel_for(const Geometry &g, bool fast, bool multi, bool timing)
 {
-    if (stream) {
-        if (packed) return fast ? (multi ? sweep_lookup_p16_f1_m1_st(C, T, NT) : sweep_lookup_p16_f1_m0_st(C, T, NT)) : sweep_lookup_p16_f0_m0_st(C, T, NT);
-        return fast ? (multi ? sweep_lookup_s32_f1_m1_st(C, T, NT) : sweep_lookup_s32_f1_m0_st(C, T, NT)) : sweep_lookup_s32_f0_m0_st(C, T, NT);
-    }
-    if (packed) return fast ? (multi ? sweep_lookup_p16_f1_m1(C, T, NT) : sweep_lookup_p16_f1_m0(C, T, NT)) : sweep_lookup_p16_f0_m0(C, T, NT);
-    return fast ? (multi ? sweep_lookup_s32_f1_m1(C, T, NT) : sweep_lookup_s32_f1_m0(C, T, NT)) : sweep_lookup_s32_f0_m0(C, T, NT);
+    // [policy: s32, p16][variant: !FAST, FAST, FAST + MULTI][symbols: staged, streamed]
+    static const SweepLookup classic[2][3][2] = {
+        {{sweep_lookup_s32_f0_m0, sweep_lookup_s32_f0_m0_st}, {sweep_lookup_s32_f1_m0, sweep_lookup_s32_f1_m0_st},
+         {sweep_lookup_s32_f1_m1, sweep_lookup_s32_f1_m1_st}},
+        {{sweep_lookup_p16_f0_m0, sweep_lookup_p16_f0_m0_st}, {sweep_lookup_p16_f1_m0, sweep_lookup_p16_f1_m0_st},
+         {sweep_lookup_p16_f1_m1, sweep_lookup_p16_f1_m1_st}}};
+    // [policy]
+    static const SweepLookup group[2] = {sweep_group_lookup_s32, sweep_group_lookup_p16};
+    // [policy][symbols]
+    static const SweepLookup lat[2][2] = {{sweep_lat_lookup_s32, sweep_lat_lookup_s32_st}, {sweep_lat_lookup_p16, sweep_lat_lookup_p16_st}};
+    const int pol = g.packed ? 1 : 0, st = g.stream ? 1 : 0;
+    if (g.lat && timing) return pol && !st ? sweep_lat_timing_lookup_p16(g) : nullptr;
+    if (g.lat) return lat[pol][st](g);
+    if (g.NG > 1) return group[pol](g);
+    return classic[pol][fast ? (multi ? 2 : 1) : 0][st](g);
 }
 
 namespace {
@@ -472,6 +483,15 @@ struct MetaView { void *p = nullptr; template <class U> U *as() { return reinter
 //   16 B), Record dense[]
 constexpr size_t OUT_HDR = 16;
 inline size_t out_counts_bytes(int nseg) { return ((size_t)nseg * 4 + 15) & ~size_t(15); }
+// Checks the header's flags (the first error in this order is reported) and returns the record total
+inline int64_t wave_total(const int *hdr)
+{
+    if (hdr[1]) throw PlanError{"CUDA: sweep timed out waiting for a partner CTA (internal error)"};
+    if (hdr[3]) throw PlanError{SD_MSG_TB_BAD_ROW};
+    if (hdr[0]) throw PlanError{"segment contains a symbol outside ACGTN"};
+    if (hdr[2] < 0) throw PlanError{"traceback overflowed its record buffer (internal error)"};
+    return hdr[2];
+}
 
 // One wave in flight: its device buffers, its layout and its events.  Two slots per device let the host->device copy of
 // wave w+1 and the device->host copy of wave w-1 run while wave w computes (three streams: in, compute, out).
@@ -527,15 +547,9 @@ public:
         const int spw = 32 / g.T;
         fast_ = (g.nslots % spw == 0) && (g.nslots / spw <= 4) && g.NS <= 15;     // 15 named barriers besides barrier 0
         if (getenv("SD_NOFAST")) fast_ = false;
-        lat_timing_ = false;
-        if (g.lat) {
-            if (g.stream) kernel_ = g.packed ? sweep_lat_lookup_p16_st(g.C, g.T, g.scanw) : sweep_lat_lookup_s32_st(g.C, g.T, g.scanw);
-            else kernel_ = g.packed ? sweep_lat_lookup_p16(g.C, g.T, g.scanw) : sweep_lat_lookup_s32(g.C, g.T, g.scanw);
-            if (getenv("SD_LAT_TIMING") && g.packed && !g.stream && sweep_lat_timing_lookup_p16(g.C, g.T, g.scanw)) { kernel_ = sweep_lat_timing_lookup_p16(g.C, g.T, g.scanw); lat_timing_ = true; }
-            if ((g.NT / 32) * g.NG > 32) throw PlanError{"internal: a deferred-jump cluster holds at most 32 warps"};
-        }
-        else kernel_ = g.NG > 1 ? (g.packed ? sweep_group_lookup_p16(g.C, g.T) : sweep_group_lookup_s32(g.C, g.T))
-                                : kern(g.packed, g.C, g.T, g.NT, fast_, fast_ && g.NS > 1, g.stream != 0);
+        lat_timing_ = g.lat && getenv("SD_LAT_TIMING") && sweep_kernel_for(g, fast_, false, true);
+        kernel_ = sweep_kernel_for(g, fast_, fast_ && g.NS > 1, lat_timing_);
+        if (g.lat && (g.NT / 32) * g.NG > 32) throw PlanError{"internal: a deferred-jump cluster holds at most 32 warps"};
         if (!kernel_) throw PlanError{"no sweep kernel compiled for this geometry"};
         cudaFuncAttributes fa;
         SD_CUDA(cudaFuncGetAttributes(&fa, kernel_));
@@ -675,25 +689,33 @@ public:
         launches += 2;
     }
 
+    // the argument fields that SweepArgs, GroupArgs and LatArgs share
+    template <class A> void fill_common_args(A &a, WaveSlot &w)
+    {
+        const Geometry &g = plan_.g;
+        a.bases = w.d_bases.as<uint8_t>(); a.seg_off = w.d_segoff.as<int64_t>(); a.nseg = w.nseg;
+        a.cta_code_off = w.d_ctacode.as<int64_t>(); a.seg_j_off = w.d_segj.as<int64_t>();
+        a.codes = w.d_codes.as<uint32_t>(); a.jr = w.d_jr.as<JR>();
+        a.slot_len = d_slotlen_.as<int>(); a.slot_endadd = d_slotend_.as<int>();
+        a.nslots = g.nslots; a.M = g.M; a.NT = g.NT; a.CW = g.CW;
+        a.ins = plan_.sc.ins; a.del = plan_.sc.del; a.deadz = plan_.deadz;
+        a.tr = g.packed ? tag_regs<Packed16>() : tag_regs<Scalar32>();
+        a.bad_symbol = w.d_out.as<int>();
+        a.rank = w.filter_on ? w.d_rank.as<int>() : nullptr;
+    }
+
     void launch_single(WaveSlot &w, int seg_stride, cudaStream_t stream)
     {
         const Geometry &g = plan_.g;
         SweepArgs a;
+        fill_common_args(a, w);
         a.prof = d_prof_.as<uint4>(); a.prof_u4 = (int)(plan_.prof.size() / 4);
-        a.bases = w.d_bases.as<uint8_t>(); a.seg_off = w.d_segoff.as<int64_t>();
-        a.nseg = w.nseg;
-        a.cta_nmax = w.d_ctanmax.as<int>(); a.cta_code_off = w.d_ctacode.as<int64_t>(); a.seg_j_off = w.d_segj.as<int64_t>();
-        a.codes = w.d_codes.as<uint32_t>(); a.jr = w.d_jr.as<JR>();
-        a.bad_symbol = w.d_out.as<int>();
-        a.rank = w.filter_on ? w.d_rank.as<int>() : nullptr;
-        a.slot_len = d_slotlen_.as<int>(); a.slot_endadd = d_slotend_.as<int>();
-        a.nslots = g.nslots; a.M = g.M; a.NS = g.NS; a.NT = g.NT; a.CW = g.CW; a.nsl = plan_.nsl; a.qp = plan_.qp;
-        a.ins = plan_.sc.ins; a.del = plan_.sc.del; a.deadz = plan_.deadz;
+        a.cta_nmax = w.d_ctanmax.as<int>();
+        a.NS = g.NS; a.nsl = plan_.nsl; a.qp = plan_.qp;
         a.seg_stride = seg_stride;
         const int spw = 32 / g.T;
         a.wps = fast_ ? g.nslots / spw : 1;
         a.kstride = fast_ ? g.NS * 4 : (g.NS + 3) / 4 * 4;
-        a.tr = g.packed ? tag_regs<Packed16>() : tag_regs<Scalar32>();
         a.scanw = getenv("SD_FULL_SCAN") ? 64 : g.scanw;
         const size_t smem = plan_.prof.size() * 4 + (size_t)3 * a.kstride * 4 + (g.stream ? 0 : (size_t)g.NS * a.seg_stride);
         if (smem > (size_t)prop_.sharedMemPerBlockOptin) throw PlanError{"sweep geometry needs more shared memory than the SM has"};
@@ -707,17 +729,11 @@ public:
     {
         const Geometry &g = plan_.g;
         GroupArgs a;
+        fill_common_args(a, w);
         a.prof = d_prof_.as<uint4>(); a.nsl_total = plan_.nsl; a.qp = plan_.qp;
-        a.bases = w.d_bases.as<uint8_t>(); a.seg_off = w.d_segoff.as<int64_t>(); a.nseg = w.nseg;
-        a.cta_code_off = w.d_ctacode.as<int64_t>(); a.seg_j_off = w.d_segj.as<int64_t>();
-        a.codes = w.d_codes.as<uint32_t>(); a.jr = w.d_jr.as<JR>();
-        a.slot_len = d_slotlen_.as<int>(); a.slot_endadd = d_slotend_.as<int>();
-        a.nslots = g.nslots; a.M = g.M; a.NT = g.NT; a.CW = g.CW; a.NG = g.NG; a.SG = g.SG; a.NS = g.NS;
-        a.ins = plan_.sc.ins; a.del = plan_.sc.del; a.deadz = plan_.deadz;
-        a.tr = g.packed ? tag_regs<Packed16>() : tag_regs<Scalar32>();
+        a.NG = g.NG; a.SG = g.SG; a.NS = g.NS;
         a.scanw = getenv("SD_FULL_SCAN") ? 64 : g.scanw;
-        a.bad_symbol = w.d_out.as<int>(); a.error = w.d_out.as<int>() + 1;
-        a.rank = w.filter_on ? w.d_rank.as<int>() : nullptr;
+        a.error = w.d_out.as<int>() + 1;
         const int spw = 32 / g.T, wps = g.NT / 32;
         const size_t sgt = (size_t)wps * spw * g.T;
         const size_t smem = (size_t)5 * sgt * plan_.qp * 16 + ((size_t)g.NS * wps + g.NS + 8) * 4;
@@ -741,19 +757,14 @@ public:
     {
         const Geometry &g = plan_.g;
         LatArgs a;
+        fill_common_args(a, w);
         a.prof2 = d_prof_.as<uint4>(); a.nsl_total = plan_.nsl; a.qp2 = plan_.qp2;
-        a.bases = w.d_bases.as<uint8_t>(); a.seg_off = w.d_segoff.as<int64_t>(); a.nseg = w.nseg;
-        a.cta_code_off = w.d_ctacode.as<int64_t>(); a.seg_j_off = w.d_segj.as<int64_t>();
-        a.codes = w.d_codes.as<uint32_t>(); a.jr = w.d_jr.as<JR>();
-        a.slot_len = d_slotlen_.as<int>(); a.slot_endadd = d_slotend_.as<int>();
-        a.nslots = g.nslots; a.M = g.M; a.NT = g.NT; a.CW = g.CW; a.NG = g.NG; a.SG = g.SG;
-        a.ins = plan_.sc.ins; a.del = plan_.sc.del; a.deadz = plan_.deadz; a.lat_th = plan_.lat_th; a.scanw = g.scanw;
+        a.NG = g.NG; a.SG = g.SG;
+        a.lat_th = plan_.lat_th; a.scanw = g.scanw;
         for (int q = 0; q < 5; ++q) a.kj[q] = plan_.kj[q];
         a.seg_kj = w.filter_on ? w.d_segkj.as<int>() : nullptr;
-        a.rank = w.filter_on ? w.d_rank.as<int>() : nullptr;
         a.seg_stride = seg_stride;
-        a.tr = g.packed ? tag_regs<Packed16>() : tag_regs<Scalar32>();
-        a.bad_symbol = w.d_out.as<int>(); a.error = w.d_out.as<int>() + 1;
+        a.error = w.d_out.as<int>() + 1;
         const int spw = 32 / g.T, wpc = g.NT / 32;
         a.dbg = nullptr;
         if (lat_timing_) { w.d_dbg.need((size_t)w.nseg * g.NG * wpc * 64); a.dbg = w.d_dbg.as<long long>(); SD_CUDA(cudaMemsetAsync(a.dbg, 0, (size_t)w.nseg * g.NG * wpc * 64, st_)); }
@@ -850,14 +861,7 @@ public:
     void finish(WaveSlot &w, BatchResult &out)
     {
         SD_CUDA(cudaEventSynchronize(w.ev[5]));
-        const int *hdr = w.h_out.as<int>();
-        if (hdr[0] || hdr[1] || hdr[3]) {
-            if (hdr[1]) throw PlanError{"CUDA: sweep timed out waiting for a partner CTA (internal error)"};
-            if (hdr[3]) throw PlanError{SD_MSG_TB_BAD_ROW};
-            throw PlanError{"segment contains a symbol outside ACGTN"};
-        }
-        const int64_t total = hdr[2];
-        if (total < 0) throw PlanError{"traceback overflowed its record buffer (internal error)"};
+        const int64_t total = wave_total(w.h_out.as<int>());
         const size_t rec_off = OUT_HDR + out_counts_bytes(w.nseg);
         const size_t base = out.recs.size();
         out.recs.resize(base + (size_t)total);
@@ -922,12 +926,10 @@ public:
         WaveSlot &w = slot_[0];
         SD_CUDA(cudaMemsetAsync(w.d_out.p, 0, OUT_HDR, st_));
         enqueue_kernels(w);
-        int flag[4] = {0, 0, 0, 0};
-        SD_CUDA(cudaMemcpyAsync(flag, w.d_out.p, OUT_HDR, cudaMemcpyDeviceToHost, st_tb_));
+        int hdr[4] = {0, 0, 0, 0};
+        SD_CUDA(cudaMemcpyAsync(hdr, w.d_out.p, OUT_HDR, cudaMemcpyDeviceToHost, st_tb_));
         SD_CUDA(cudaStreamSynchronize(st_tb_));
-        if (flag[1]) throw PlanError{"CUDA: sweep timed out waiting for a partner CTA (internal error)"};
-        if (flag[3]) throw PlanError{SD_MSG_TB_BAD_ROW};
-        if (flag[0]) throw PlanError{"segment contains a symbol outside ACGTN"};
+        wave_total(hdr);                  // the records are compacted by fetch(): the total is still 0 here
         float ms = 0;
         SD_CUDA(cudaEventElapsedTime(&ms, w.ev[2], w.ev[3])); sweep_ms += ms;
         SD_CUDA(cudaEventElapsedTime(&ms, w.ev[6], w.ev[4])); traceback_ms += ms;

@@ -120,11 +120,7 @@ __global__ void sweep_lat_kernel(const LatArgs a)
         const int row = min((NG > 1 ? grp * a.SG * T : 0) + r / a.qp2, a.nsl_total - 1);
         sprof[x] = a.prof2[((size_t)sym * a.nsl_total + row) * a.qp2 + (r % a.qp2)];
     }
-    for (int x = tid; x < (ST ? 0 : a.seg_stride); x += NT) {
-        int code = (x < n) ? ascii_code(a.bases[o + x]) : 0;
-        if (code > 4) { *a.bad_symbol = 1; code = 0; }
-        schar[x] = (uint8_t)code;
-    }
+    for (int x = tid; x < (ST ? 0 : a.seg_stride); x += NT) schar[x] = (uint8_t)((x < n) ? symbol_code(a.bases[o + x], a.bad_symbol) : 0);
     if (tid < 5) skj[tid] = a.seg_kj ? a.seg_kj[(size_t)seg * 5 + tid] : a.kj[tid];
     for (int x = tid; x < LAT_NBUF * 32; x += NT) xkey[x] = 0ull;            // column tag 0 = nothing published
     __syncthreads();
@@ -137,16 +133,9 @@ __global__ void sweep_lat_kernel(const LatArgs a)
     const bool kill_first = (t == 0), kill_last = (t == T - 1 && L == 1);
     const bool is_end = active && t == T - 1;
     const bool j_writer = grp == 0 && tid == 0;
-    int tb_lo = slot, tb_hi = a.M + slot;
-    if (a.rank && active) {
-        const int *rk = a.rank + (size_t)seg * (2 * a.M);
-        tb_lo = rk[slot]; tb_hi = (P::ROWS == 2) ? rk[a.M + slot] : -1;
-    }
     // key = (half << 10) + const: the row-end word is U (tag 2: 0x800 too much) in column 0, g (tag 3: 0xC00) afterwards
-    const bool key_lo = is_end && tb_lo >= 0;
-    const int kc_lo = key_lo ? key_const(endadd, tb_lo) : SD_KEY_NONE;
-    const int kc_hi = (is_end && tb_hi >= 0) ? key_const(endadd, tb_hi) : SD_KEY_NONE;
-    const int kc3_lo = kc_lo - 0xC00, kc3_hi = kc_hi - 0xC00;
+    const SlotKey sk = slot_key<P>(active, is_end, endadd, slot, a.M, a.rank, seg, 0, 0);
+    const int kc3_lo = sk.kc_lo - 0xC00, kc3_hi = sk.kc_hi - 0xC00;
     JR *jptr = a.jr + a.seg_j_off[seg];
     uint32_t *cptr = a.codes + a.cta_code_off[(size_t)seg * NG + grp] + (size_t)tid * a.CW;
     const size_t cstride = (size_t)NT * a.CW;
@@ -222,31 +211,18 @@ __global__ void sweep_lat_kernel(const LatArgs a)
     constexpr int NW = (C + P::CELLS_PER_WORD - 1) / P::CELLS_PER_WORD;
     uint32_t cw[NW];
     auto store_codes = [&]() {
-        if (active) {
-            if (NW == 2) *reinterpret_cast<uint2 *>(cptr) = make_uint2(cw[0], cw[1]);
-            else if (NW == 4) *reinterpret_cast<uint4 *>(cptr) = make_uint4(cw[0], cw[1], cw[2], cw[3]);
-            else {
-#pragma unroll
-                for (int w = 0; w < NW; ++w) cptr[w] = cw[w];
-            }
-        }
+        if (active) store_code_words(cptr, cw);
         cptr += cstride;
     };
 
     // ST: symbols past the end of the segment read as 0, like the 0-padded buffer
-    auto symbol = [&](int i) {
-        int code = (i < n) ? ascii_code(__ldg(a.bases + o + i)) : 0;
-        if (code > 4) { *a.bad_symbol = 1; code = 0; }
-        return code;
-    };
+    auto symbol = [&](int i) { return (i < n) ? symbol_code(__ldg(a.bases + o + i), a.bad_symbol) : 0; };
 
     // ---- column 0 in the classic form: its jump base (row-0 rule, main.cpp:171-182) needs no exchange -------------
 #pragma unroll
     for (int kk = 0; kk < C; ++kk) X[kk] = deadu;
     load_p(myprof + (ST ? symbol(0) : schar[0]) * sym_stride);
-    if (t == 0 && L > 1) pw[0] = P::add(pw[0], P::splat(4 * a.del));
-    if (t == T - 1 && L == 1) pw[C - 1] = P::add(pw[C - 1], P::splat(4 * a.del));
-    lane_pre<P, C>(X, deadu, pw, deadu, kill_first, kill_last);
+    lane_pre_col0<P, C>(X, pw, a.del, L, deadu, kill_first, kill_last);
     {
         const uint32_t E = lane_post<P, C>(X, pw, P::splat(1), deadu, tr);
         const uint32_t carry = window_carry<P, T, 0>(E, t, deadu);
@@ -256,10 +232,8 @@ __global__ void sweep_lat_kernel(const LatArgs a)
         uint32_t ufirst;
         const uint32_t uend = lane_pass2_pre<P, C>(X, carry, cw, tr, pw, deadu, kill_last, &ufirst);
         store_codes();
-        publish(0u, 1, __reduce_max_sync(0xffffffffu, lane_key<P>(uend, kc_lo, kc_hi, key_lo, 0x800)));
-        uint32_t prevU = deadu;
-        if (T > 1) { prevU = __shfl_up_sync(0xffffffffu, uend, 1); if (t == 0) prevU = deadu; }
-        X[0] = lane_pre_first<P>(prevU, pw[0], ufirst, deadu, kill_first, C == 1 && kill_last);
+        publish(0u, 1, __reduce_max_sync(0xffffffffu, lane_key<P>(uend, sk.kc_lo, sk.kc_hi, sk.counted, 0x800)));
+        X[0] = next_first_cell<P, C, T>(uend, pw[0], ufirst, deadu, t, kill_first, kill_last);
     }
 
     int jbase = a.ins;            // Bref + (i-1)*ins when J[i] is formed
@@ -294,7 +268,7 @@ __global__ void sweep_lat_kernel(const LatArgs a)
         load_p(pn);                                       // flies during the chain
         const uint32_t g = lat_chain<P, C>(X, carry, trr);
         tick(1);
-        publish(boff, i + 1, __reduce_max_sync(0xffffffffu, lane_key<P, true>(g, kc3_lo, kc3_hi, key_lo)));
+        publish(boff, i + 1, __reduce_max_sync(0xffffffffu, lane_key<P, true>(g, kc3_lo, kc3_hi, sk.counted)));
         tick(2);
 
         // J[i] from the key of column i-1, published one column ago
@@ -347,13 +321,13 @@ __global__ void sweep_lat_kernel(const LatArgs a)
 }
 
 // WN: carry window the kernel is compiled for (0 = any, log-depth scan)
-const void *sweep_lat_lookup_p16(int C, int T, int W);
-const void *sweep_lat_lookup_s32(int C, int T, int W);
-const void *sweep_lat_lookup_p16_st(int C, int T, int W);                 // ST: symbols streamed from global memory
-const void *sweep_lat_lookup_s32_st(int C, int T, int W);
-const void *sweep_lat_timing_lookup_p16(int C, int T, int W);            // instrumented twins (SD_LAT_TIMING=1, exploration only)
+const void *sweep_lat_lookup_p16(const Geometry &g);
+const void *sweep_lat_lookup_s32(const Geometry &g);
+const void *sweep_lat_lookup_p16_st(const Geometry &g);                  // ST: symbols streamed from global memory
+const void *sweep_lat_lookup_s32_st(const Geometry &g);
+const void *sweep_lat_timing_lookup_p16(const Geometry &g);             // instrumented twins (SD_LAT_TIMING=1, exploration only)
 
-// smallest compiled window >= W
+// smallest compiled window >= W (= g.scanw)
 #define SD_LAT_PICK(POLICY, CC, TT, TMF, STF)                                                                        \
     if (C == CC && T == TT) {                                                                                         \
         if (W <= 2) return (const void *)sweep_lat_kernel<POLICY, CC, TT, 2, TMF, STF>;                               \
@@ -363,8 +337,9 @@ const void *sweep_lat_timing_lookup_p16(int C, int T, int W);            // inst
     }
 
 #define SD_INSTANTIATE_LAT(NAME, POLICY, STF)                                                                        \
-    const void *NAME(int C, int T, int W)                                                                             \
+    const void *NAME(const Geometry &g)                                                                               \
     {                                                                                                                 \
+        const int C = g.C, T = g.T, W = g.scanw;                                                                      \
         SD_LAT_PICK(POLICY, 6, 32, false, STF) SD_LAT_PICK(POLICY, 12, 16, false, STF)                                \
         SD_LAT_PICK(POLICY, 12, 32, false, STF) SD_LAT_PICK(POLICY, 24, 8, false, STF)                                \
         SD_LAT_PICK(POLICY, 24, 16, false, STF) SD_LAT_PICK(POLICY, 24, 32, false, STF)                               \

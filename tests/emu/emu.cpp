@@ -16,7 +16,7 @@ namespace sdb {
 
 namespace {
 
-bool &bad_symbol() { static thread_local bool f = false; return f; }
+int &bad_symbol() { static thread_local int f = 0; return f; }
 bool &window_violation() { static thread_local bool f = false; return f; }
 bool &key_violation() { static thread_local bool f = false; return f; }
 
@@ -62,8 +62,7 @@ void emu_cta(const Plan &p, const Batch &b, int seg_first, int nseg_cta, int nma
         return l;
     };
     auto load_profile = [&](int tid, const LaneId &l, int i) {
-        int sym = (i < l.n) ? ascii_code(b.text[b.off[seg_first + l.seg_local] + i]) : 0;
-        if (sym > 4) { bad_symbol() = true; sym = 0; }
+        const int sym = (i < l.n) ? symbol_code(b.text[b.off[seg_first + l.seg_local] + i], &bad_symbol()) : 0;
         for (int kk = 0; kk < C; ++kk)
             PW[tid][kk] = p.prof[(((size_t)sym * p.nsl + l.sl) * p.qp + kk / 4) * 4 + (kk % 4)];
     };
@@ -72,9 +71,7 @@ void emu_cta(const Plan &p, const Batch &b, int seg_first, int nseg_cta, int nma
         const LaneId l = lane_id(tid);
         const int L = p.slot_len[l.slot];
         load_profile(tid, l, 0);
-        if (l.t == 0 && L > 1) PW[tid][0] = P::add(PW[tid][0], P::splat(4 * p.sc.del));
-        if (l.t == T - 1 && L == 1) PW[tid][C - 1] = P::add(PW[tid][C - 1], P::splat(4 * p.sc.del));
-        lane_pre<P, C>(X[tid], deadu, PW[tid], deadu, l.t == 0, l.t == T - 1 && L == 1);
+        lane_pre_col0<P, C>(X[tid], PW[tid], p.sc.del, L, deadu, l.t == 0, l.t == T - 1 && L == 1);
     }
     std::vector<uint32_t> ufirst(NT), uend(NT);
     for (int i = 0;; ++i) {
@@ -113,10 +110,8 @@ void emu_cta(const Plan &p, const Batch &b, int seg_first, int nseg_cta, int nma
             }
             // the kernels' key of every lane (an idle lane counts towards the segment of its warp, as in the warp reduction)
             if (l.seg_local < nseg_cta) {
-                const int endadd = p.slot_endadd[l.slot];
-                const int kc_lo = (is_end && row_lo >= 0) ? key_const(endadd, row_lo) - 0x800 : SD_KEY_NONE;
-                const int kc_hi = (is_end && row_hi >= 0) ? key_const(endadd, row_hi) - 0x800 : SD_KEY_NONE;
-                dkey[l.seg_local] = std::max(dkey[l.seg_local], lane_key<P>(u, kc_lo, kc_hi, is_end && row_lo >= 0));
+                const SlotKey sk = slot_key<P>(l.active, is_end, p.slot_endadd[l.slot], l.slot, g.M, rank, 0, l.seg_local, -0x800);
+                dkey[l.seg_local] = std::max(dkey[l.seg_local], lane_key<P>(u, sk.kc_lo, sk.kc_hi, sk.counted));
             }
         }
         for (int s = 0; s < nseg_cta; ++s)
@@ -179,11 +174,7 @@ void emu_cta_lat(const Plan &p, const Batch &b, int seg_first, int nseg_cta, int
         l.sl = l.slot * T + l.t;
         return l;
     };
-    auto symbol = [&](int i) {
-        int sym = (i < n) ? ascii_code(b.text[b.off[seg_first] + i]) : 0;
-        if (sym > 4) { bad_symbol() = true; sym = 0; }
-        return sym;
-    };
+    auto symbol = [&](int i) { return (i < n) ? symbol_code(b.text[b.off[seg_first] + i], &bad_symbol()) : 0; };
     auto load_profile = [&](int tid, const LaneId &l, int i) {
         const uint32_t *row = p.prof2.data() + (((size_t)symbol(i) * p.nsl + l.sl) * p.qp2) * 4;
         for (int kk = 0; kk < C; ++kk) { PW[tid][kk] = row[kk]; PT[tid][kk] = row[C + kk]; }
@@ -200,18 +191,14 @@ void emu_cta_lat(const Plan &p, const Batch &b, int seg_first, int nseg_cta, int
         const LaneId l = lane_id(tid);
         const int L = p.slot_len[l.slot];
         load_profile(tid, l, 0);
-        if (l.t == 0 && L > 1) PW[tid][0] = P::add(PW[tid][0], P::splat(4 * p.sc.del));
-        if (l.t == T - 1 && L == 1) PW[tid][C - 1] = P::add(PW[tid][C - 1], P::splat(4 * p.sc.del));
-        lane_pre<P, C>(X[tid], deadu, PW[tid], deadu, l.t == 0, l.t == T - 1 && L == 1);
+        lane_pre_col0<P, C>(X[tid], PW[tid], p.sc.del, L, deadu, l.t == 0, l.t == T - 1 && L == 1);
         E[tid] = lane_post<P, C>(X[tid], PW[tid], P::splat(0 + 1), deadu, tr);
     }
     for (int tid = 0; tid < NT; ++tid) carry[tid] = (lane_id(tid).t == 0) ? deadu : P::max2(carry[tid - 1], E[tid - 1]);
     // the kernel's key of a lane (sweep_lat_kernel: kc_lo / kc3_lo); tag_off 0x800 in column 0, 0xC00 afterwards
     auto device_key = [&](const LaneId &l, uint32_t u, int tag_off, auto floor) {
-        const bool is_end = l.active && l.t == T - 1;
-        const int kc_lo = (is_end && tie_lo(l) >= 0) ? key_const(p.slot_endadd[l.slot], tie_lo(l)) : SD_KEY_NONE;
-        const int kc_hi = (is_end && tie_hi(l) >= 0) ? key_const(p.slot_endadd[l.slot], tie_hi(l)) : SD_KEY_NONE;
-        return lane_key<P, decltype(floor)::value>(u, kc_lo, kc_hi, is_end && tie_lo(l) >= 0, tag_off);
+        const SlotKey sk = slot_key<P>(l.active, l.active && l.t == T - 1, p.slot_endadd[l.slot], l.slot, g.M, rank, 0, 0, 0);
+        return lane_key<P, decltype(floor)::value>(u, sk.kc_lo, sk.kc_hi, sk.counted, tag_off);
     };
     int kpub = INT_MIN;                                  // key published for the column just swept
     int dkey = INT_MIN;
@@ -365,7 +352,7 @@ public:
         jr_.assign((size_t)lay_.seg_j_off.back(), JR{0, 0});
         const int nseg = s1_ - s0_, nctas = (int)lay_.cta_nmax.size();
         EmuFlags::overflow() = false;
-        bad_symbol() = false;
+        bad_symbol() = 0;
         const int nunits = g.NG > 1 ? nseg : nctas;          // group mode: one emulated unit per segment (all its CTAs)
         for (int c = 0; c < nunits; ++c) {
             int first = g.NG > 1 ? c : c * g.NS, cnt = g.NG > 1 ? 1 : std::min(g.NS, nseg - first);
