@@ -128,8 +128,9 @@ public:
     virtual void collect(int slot, BatchResult &out) { (void)slot; fetch(out); }
     double sweep_ms = 0, traceback_ms = 0, h2d_ms = 0, d2h_ms = 0;     // accumulated since reset_stats()
     int64_t h2d_bytes = 0, d2h_bytes = 0, launches = 0;
+    int group_slots = 0;            // group sweep: most slot groups (CTA groups that loop over segment blocks) of a launch
     int ed_thr_ = -1;
-    void reset_stats() { sweep_ms = traceback_ms = h2d_ms = d2h_ms = 0; h2d_bytes = d2h_bytes = launches = 0; }
+    void reset_stats() { sweep_ms = traceback_ms = h2d_ms = d2h_ms = 0; h2d_bytes = d2h_bytes = launches = 0; group_slots = 0; }
 };
 
 // rank tables of the pre-filter for one segment: rows sorted by (distance, row); the first one and every row with

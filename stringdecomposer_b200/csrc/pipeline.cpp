@@ -403,8 +403,8 @@ void Engine::decompose(const Batch &b, BatchResult &out)
                 else if (w >= 1) dev.collect((int)((w - 1) % (size_t)nsl), part[d]);
             }
             if (nsl > 1 && !waves.empty()) dev.collect((int)((waves.size() - 1) % (size_t)nsl), part[d]);
-            if (prof) fprintf(stderr, "[sd_b200 profile] dev %d: %zu wave(s), segments [%d,%d): %.3f ms host wall (sweep %.3f traceback %.3f h2d %.3f ms on the device)\n",
-                              d, waves.size(), bounds[d], s_end, ms(t0, now()), dev.sweep_ms, dev.traceback_ms, dev.h2d_ms);
+            if (prof) fprintf(stderr, "[sd_b200 profile] dev %d: %zu wave(s), segments [%d,%d): %.3f ms host wall (sweep %.3f traceback %.3f h2d %.3f ms on the device), %d group slot(s)\n",
+                              d, waves.size(), bounds[d], s_end, ms(t0, now()), dev.sweep_ms, dev.traceback_ms, dev.h2d_ms, dev.group_slots);
         } catch (PlanError &e) { errs[d] = e.msg.empty() ? "error" : e.msg; }
         catch (std::exception &e) { errs[d] = e.what(); }
     };

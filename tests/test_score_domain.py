@@ -22,7 +22,8 @@ import sd_oracle
 from stringdecomposer_b200 import Decomposer, SdError
 
 SD_ERR_UNSUPPORTED, SD_ERR_INTERNAL = 3, 5
-ENV_KEYS = ("SD_LAT", "SD_LAT_WARPS", "SD_GROUP_SLOTS", "SD_STREAM_SYMBOLS", "SD_FORCE_S32", "SD_GEOM", "SD_EMU_BAD_JUMP_ROW")
+ENV_KEYS = ("SD_LAT", "SD_LAT_WARPS", "SD_GROUP_SLOTS", "SD_GROUP_GSLOTS", "SD_STREAM_SYMBOLS", "SD_FORCE_S32", "SD_GEOM",
+            "SD_EMU_BAD_JUMP_ROW", "SD_WAVE_BYTES", "SD_PROFILE")
 _AL = np.frombuffer(b"ACGT", dtype=np.uint8)
 
 
