@@ -33,24 +33,22 @@
 
 #define SDO_NEG_INF (-1000000) /* main.cpp:156 "INF" */
 
-/* ---------------------------------------------------------------------------------------
- * One segment against all DP rows.  Restates MonomersAligner::AlignPartClassicDP,
- * main.cpp:151-270: allocation :158-169, row 0 :171-182, sweep :183-208, final argmax
- * :209-216, equality-test traceback :217-267, reversal :268.
- * rows: concatenated row strings (forward monomers then reverse complements), row r occupies
- * rows[row_off[r] .. row_off[r+1]).  Output records are in read order, positions relative to
- * the segment.  Returns the record count, or -1 if out is too small / allocation failed.
- * ------------------------------------------------------------------------------------- */
-int sdo_align_segment(const char *seg, int n, const char *rows, const int *row_off, int R,
-                      int ins, int del, int mismatch, int match, sdo_rec *out, int cap)
-{
-    if (n <= 0 || R <= 0) return 0;
-    const int64_t width = row_off[R];           /* total cells of one column */
-    int64_t *tab = (int64_t *)malloc(sizeof(int64_t) * (size_t)n * (size_t)width);
-    int64_t *jump = (int64_t *)malloc(sizeof(int64_t) * (size_t)n); /* dp[i][monomers_num][0] */
-    if (!tab || !jump) { free(tab); free(jump); return -1; }
 #define CELL(i, r, k) tab[(int64_t)(i) * width + row_off[r] + (k)]
 #define ROWLEN(r) (row_off[(r) + 1] - row_off[r])
+
+/* ---------------------------------------------------------------------------------------
+ * The forward DP of one segment against all DP rows: allocation main.cpp:158-169, row 0 :171-182, sweep :183-208.
+ * rows: concatenated row strings (forward monomers then reverse complements), row r occupies
+ * rows[row_off[r] .. row_off[r+1]).  Returns the flat table (cell (i, r, k) at i*row_off[R] + row_off[r] + k) and
+ * sets *jump_out to jump[i] = dp[i][monomers_num][0]; both malloc'd.  NULL if an allocation failed.
+ * ------------------------------------------------------------------------------------- */
+static int64_t *fill_table(const char *seg, int n, const char *rows, const int *row_off, int R,
+                           int ins, int del, int mismatch, int match, int64_t **jump_out)
+{
+    const int64_t width = row_off[R];           /* total cells of one column */
+    int64_t *tab = (int64_t *)malloc(sizeof(int64_t) * (size_t)n * (size_t)width);
+    int64_t *jump = (int64_t *)malloc(sizeof(int64_t) * (size_t)n);
+    if (!tab || !jump) { free(tab); free(jump); return NULL; }
     for (int64_t x = 0; x < (int64_t)n * width; ++x) tab[x] = SDO_NEG_INF;       /* :160-166 */
     for (int i = 0; i < n; ++i) jump[i] = SDO_NEG_INF;                            /* :167-168 */
 
@@ -100,6 +98,25 @@ int sdo_align_segment(const char *seg, int n, const char *rows, const int *row_o
             }
         }
     }
+    *jump_out = jump;
+    return tab;
+}
+
+/* ---------------------------------------------------------------------------------------
+ * One segment against all DP rows.  Restates MonomersAligner::AlignPartClassicDP,
+ * main.cpp:151-270: forward DP (fill_table) :156-208, final argmax :209-216, equality-test traceback :217-267,
+ * reversal :268.  Output records are in read order, positions relative to the segment.  Returns the record count,
+ * or -1 if out is too small / allocation failed.
+ * ------------------------------------------------------------------------------------- */
+int sdo_align_segment(const char *seg, int n, const char *rows, const int *row_off, int R,
+                      int ins, int del, int mismatch, int match, sdo_rec *out, int cap)
+{
+    if (n <= 0 || R <= 0) return 0;
+    const int64_t width = row_off[R];
+    int64_t *jump = NULL;
+    int64_t *tab = fill_table(seg, n, rows, row_off, R, ins, del, mismatch, match, &jump);
+    if (!tab) return -1;
+
     /* final argmax, main.cpp:209-216: int max_score, strict '<', lowest row wins */
     int top = SDO_NEG_INF, top_row = R;
     for (int r = 0; r < R; ++r) {
@@ -159,12 +176,54 @@ int sdo_align_segment(const char *seg, int n, const char *rows, const int *row_o
         }
     }
     free(tab); free(jump);
-#undef CELL
-#undef ROWLEN
     if (fail) return -1;
     for (int a = 0, b = cnt - 1; a < b; ++a, --b) { sdo_rec t = out[a]; out[a] = out[b]; out[b] = t; } /* :268 */
     return cnt;
 }
+
+/* ---------------------------------------------------------------------------------------
+ * The DP table of one segment as the reference's traceback reads it (main.cpp:217-267), cell by cell:
+ *   code[i * row_off[R] + row_off[r] + k]: the move the traceback takes at (i, r, k), in the order of :242-253:
+ *     0 the deletion equality holds (k != 0), else 1 the insertion equality (i != 0; no k guard, :245), else 2 the
+ *     diagonal equality (i != 0, k != 0), else 3 (close the alignment)
+ *   J[i], i = 1..n-1: jump[i] = max_r dp[i-1][r][last];  J[n]: the final maximum (:209-216)
+ *   argJ[i]: the lowest row attaining J[i] -- the row the jump state picks (:230-236); argJ[n] = top row (:212)
+ * J[0] and argJ[0] are set to 0.  Returns 0, or -1 if an allocation failed.
+ * ------------------------------------------------------------------------------------- */
+int sdo_dp_tables(const char *seg, int n, const char *rows, const int *row_off, int R,
+                  int ins, int del, int mismatch, int match, int8_t *code, int64_t *J, int *argJ)
+{
+    if (n <= 0 || R <= 0) return 0;
+    const int64_t width = row_off[R];
+    int64_t *jump = NULL;
+    int64_t *tab = fill_table(seg, n, rows, row_off, R, ins, del, mismatch, match, &jump);
+    if (!tab) return -1;
+    for (int i = 0; i < n; ++i)
+        for (int r = 0; r < R; ++r) {
+            const char *m = rows + row_off[r];
+            for (int k = 0; k < ROWLEN(r); ++k) {
+                const int64_t h = CELL(i, r, k);
+                const int sub = (m[k] == seg[i]) ? match : mismatch;
+                int c = 3;
+                if (k != 0 && h == CELL(i, r, k - 1) + del) c = 0;                                /* :242 */
+                else if (i != 0 && h == CELL(i - 1, r, k) + ins) c = 1;                           /* :245 */
+                else if (i != 0 && k != 0 && h == CELL(i - 1, r, k - 1) + sub) c = 2;             /* :249 */
+                code[(int64_t)i * width + row_off[r] + k] = (int8_t)c;
+            }
+        }
+    J[0] = 0; argJ[0] = 0;
+    for (int i = 1; i <= n; ++i) {
+        J[i] = SDO_NEG_INF; argJ[i] = R;
+        for (int r = 0; r < R; ++r) {
+            const int64_t e = CELL(i - 1, r, ROWLEN(r) - 1);
+            if (e > J[i]) { J[i] = e; argJ[i] = r; }                                     /* strict: lowest row */
+        }
+    }
+    free(tab); free(jump);
+    return 0;
+}
+#undef CELL
+#undef ROWLEN
 
 /* ---------------------------------------------------------------------------------------
  * MonomerEditDistance, main.cpp:128-133: edlibAlign(monomer, segment, k = -1, EDLIB_MODE_HW,

@@ -3,6 +3,7 @@
 #ifndef SD_ORACLE_H
 #define SD_ORACLE_H
 #include <stddef.h>
+#include <stdint.h>
 #include <stdio.h>
 #ifdef __cplusplus
 extern "C" {
@@ -14,6 +15,8 @@ typedef struct { int row; int start; int end; float score; } sdo_rec;
 
 int sdo_align_segment(const char *seg, int n, const char *rows, const int *row_off, int R,
                       int ins, int del, int mismatch, int match, sdo_rec *out, int cap);
+int sdo_dp_tables(const char *seg, int n, const char *rows, const int *row_off, int R,
+                  int ins, int del, int mismatch, int match, int8_t *code, int64_t *J, int *argJ);
 int sdo_segment_read(long read_len, int part_size, int overlap, int *offs, int *lens, int cap);
 int sdo_postprocess(const sdo_rec *in, int n, sdo_rec *out);
 int sdo_hw_distance(const char *query, int m, const char *target, int n);

@@ -31,6 +31,9 @@ def lib():
         _lib.sdo_align_segment.argtypes = [C.c_char_p, C.c_int, C.c_char_p, C.POINTER(C.c_int), C.c_int, C.c_int, C.c_int,
                                            C.c_int, C.c_int, C.POINTER(Rec), C.c_int]
         _lib.sdo_align_segment.restype = C.c_int
+        _lib.sdo_dp_tables.argtypes = [C.c_char_p, C.c_int, C.c_char_p, C.POINTER(C.c_int), C.c_int, C.c_int, C.c_int, C.c_int,
+                                       C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
+        _lib.sdo_dp_tables.restype = C.c_int
         _lib.sdo_segment_read.argtypes = [C.c_long, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_int]
         _lib.sdo_segment_read.restype = C.c_int
         _lib.sdo_postprocess.argtypes = [C.POINTER(Rec), C.c_int, C.POINTER(Rec)]
@@ -75,6 +78,33 @@ def align_segment(seg, monomers, scoring=(-1, -1, -1, 1), ed_thr=-1):
     if n < 0:
         raise RuntimeError("oracle failed (%d)" % n)
     return [(keep[out[i].row], out[i].start, out[i].end, out[i].score) for i in range(n)]
+
+
+def dp_tables(seg, monomers, scoring=(-1, -1, -1, 1), ed_thr=-1):
+    """The DP table of one segment as the reference's traceback reads it (main.cpp:217-267) -> dict of numpy arrays:
+      code  int8 [n][row_off[R]]: the traceback's move at cell (i, r, k) = code[i, row_off[r] + k]: 0 deletion,
+            1 insertion, 2 diagonal, 3 close the alignment (the first equality of main.cpp:242-253 that holds)
+      J     int64 [n+1]: J[i] = max_r H[i-1][r][last] for i = 1..n (J[n] is the final maximum)
+      argJ  int32 [n+1]: the lowest row attaining J[i] (argJ[n] is the top row)
+      row_off int32 [R+1], keep: the rows of the table as indices into rows_of(monomers).  With ed_thr > -1 the table
+            covers the rows that FilterMonomersForRead keeps, in rank order, as align_segment does."""
+    import numpy as np
+    rows = rows_of(monomers)
+    keep = list(range(len(rows)))
+    if ed_thr > -1:
+        keep = filter_rows(seg, rows, ed_thr)
+        rows = [rows[k] for k in keep]
+    n = len(seg)
+    ro = np.zeros(len(rows) + 1, np.int32)
+    ro[1:] = np.cumsum([len(r) for r in rows])
+    code = np.zeros((n, int(ro[-1])), np.int8)
+    J = np.zeros(n + 1, np.int64)
+    argJ = np.zeros(n + 1, np.int32)
+    st = lib().sdo_dp_tables(seg.encode(), n, "".join(rows).encode(), ro.ctypes.data_as(C.POINTER(C.c_int)), len(rows),
+                             scoring[0], scoring[1], scoring[2], scoring[3], code.ctypes.data, J.ctypes.data, argJ.ctypes.data)
+    if st < 0:
+        raise RuntimeError("oracle failed (%d)" % st)
+    return {"code": code, "J": J, "argJ": argJ, "row_off": ro, "keep": keep}
 
 
 def segment_read(read_len, part, overlap):

@@ -101,6 +101,12 @@ struct CtaLayout {
     std::vector<int64_t> seg_rec_off;    // scratch record offset of each segment (cap = n) (+1 sentinel)
 };
 CtaLayout make_cta_layout(const Plan &p, const Batch &b, int seg_begin, int seg_end);
+// SD_DUMP_TABLES=<directory> (tests): the directory into which every wave's sweep output is written, or null.
+// dump_wave_tables writes one wave as <directory>/wave_<first segment, 8 digits>.bin (little-endian):
+//   int32 packed, C, T, nslots, M, NS, NT, CW, NG, SG, lat, scanw, stream (Geometry), first segment, nseg, nctas;
+//   int64 cta_code_off[nctas + 1], seg_j_off[nseg + 1]; uint32 codes[cta_code_off[nctas]]; int32 {j, row}[seg_j_off[nseg]]
+const char *dump_tables_dir();
+void dump_wave_tables(const char *dir, const Geometry &g, int first, const CtaLayout &l, const uint32_t *codes, const JR *jr);
 
 // Backend interface.  configure() binds a plan; stage() copies a range of segments to the device;
 // execute() runs sweep + traceback with inputs and outputs resident; fetch() brings the records back.

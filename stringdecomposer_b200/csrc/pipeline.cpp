@@ -306,6 +306,29 @@ void Engine::note_split(const Batch &b, const std::vector<int> &bounds)
     }
 }
 
+const char *dump_tables_dir()
+{
+    const char *e = getenv("SD_DUMP_TABLES");
+    return e && *e ? e : nullptr;
+}
+
+void dump_wave_tables(const char *dir, const Geometry &g, int first, const CtaLayout &l, const uint32_t *codes, const JR *jr)
+{
+    const int nseg = (int)l.seg_j_off.size() - 1, nctas = (int)l.cta_code_off.size() - 1;
+    const int32_t hdr[16] = {g.packed, g.C, g.T, g.nslots, g.M, g.NS, g.NT, g.CW, g.NG, g.SG, g.lat, g.scanw, g.stream, first, nseg, nctas};
+    char name[64];
+    snprintf(name, sizeof name, "/wave_%08d.bin", first);
+    const std::string path = std::string(dir) + name;
+    FILE *f = fopen(path.c_str(), "wb");
+    bool ok = f && fwrite(hdr, sizeof hdr, 1, f) == 1 &&
+              fwrite(l.cta_code_off.data(), 8, l.cta_code_off.size(), f) == l.cta_code_off.size() &&
+              fwrite(l.seg_j_off.data(), 8, l.seg_j_off.size(), f) == l.seg_j_off.size() &&
+              fwrite(codes, 4, (size_t)l.cta_code_off.back(), f) == (size_t)l.cta_code_off.back() &&
+              fwrite(jr, sizeof(JR), (size_t)l.seg_j_off.back(), f) == (size_t)l.seg_j_off.back();
+    if (f && fclose(f) != 0) ok = false;
+    if (!ok) throw PlanError{"SD_DUMP_TABLES: cannot write " + path};
+}
+
 // contiguous, column-balanced ranges, one per device (SURVEY 8e: segments are independent, no collective)
 void Engine::split(const Batch &b, std::vector<int> &bounds) const
 {

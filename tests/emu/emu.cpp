@@ -402,6 +402,7 @@ public:
                                         recs_.data() + lay_.seg_rec_off[s], n, true,
                                         r2r_.empty() ? nullptr : r2r_.data() + (size_t)s * ms_.nrows(), ms_.nrows());
         }
+        if (const char *dir = dump_tables_dir()) dump_wave_tables(dir, g, s0_, lay_, codes_.data(), jr_.data());
     }
     void fetch(BatchResult &out) override
     {

@@ -34,7 +34,8 @@ def problems(draw):
     return monomers, segments, scoring, geom, group, lat
 
 
-def run(flavour, problem):
+def problem_env(problem):
+    """the test overrides of a problem (an empty value: unset)"""
     monomers, segments, scoring, geom, group, lat = problem
     lmax = max(len(m) for m in monomers)
     if geom:
@@ -45,6 +46,12 @@ def run(flavour, problem):
     if "," in lat:
         c, t, w = lat.split(",")
         env.update({"SD_LAT": "1", "SD_GEOM": "%s,%s,1" % (c, t), "SD_LAT_WARPS": w, "SD_GROUP_SLOTS": ""})
+    return env
+
+
+def run(flavour, problem):
+    monomers, segments, scoring, geom, group, lat = problem
+    env = problem_env(problem)
     for k, v in env.items():
         if v:
             os.environ[k] = v
