@@ -17,6 +17,8 @@
  *     the full matrix.  Above 1 MiB of traceback state edlib switches to Hirschberg splitting
  *     (edlib.cpp:1189-1191), which may choose another optimal path: sdo_nw_uses_traceback() says which side
  *     a pair is on; the pinning below only covers the traceback side.
+ * sdo_nw_prefix_counts gives the triple of every prefix pair from one matrix (for the cell-by-cell tests of the
+ * kernel, tests/test_identity_tables.py) and sdo_nw_path_counts_batch runs the walk over a pair list in parallel.
  * Parity: PINNED -- against the reference's own edlib.cpp compiled into oracle/_ref/libedlib_ref.so
  * (tests/test_identity_oracle.py, random and adversarial pairs) and, through oracle/sd_convert_oracle.py,
  * against all 12 columns of the reference's golden file test_data/final_decomposition_fc89af8.tsv. */
@@ -31,15 +33,12 @@ int sdo_nw_uses_traceback(int qlen, int tlen)
     return bytes < 1024 * 1024;
 }
 
-/* Returns the edit distance; *matches = number of '=' columns, *columns = alignment length.
- * Either sequence empty: main.py:30-33 returns (-1, "") -> identity 0; reported here as -1. */
-int sdo_nw_path_counts(const char *q, int qlen, const char *t, int tlen, int *matches, int *columns)
+/* The unit-cost NW matrix with its boundary: a (qlen+1) x (tlen+1) table, D[i][j] at [(i+1)*(tlen+1) + j+1]. */
+static int *nw_matrix(const char *q, int qlen, const char *t, int tlen)
 {
-    *matches = 0; *columns = 0;
-    if (qlen <= 0 || tlen <= 0) return -1;
     size_t W = (size_t)tlen + 1;
     int *D = (int *)malloc(sizeof(int) * (size_t)(qlen + 1) * W);
-    if (!D) return -2;
+    if (!D) return NULL;
 #define AT(i, j) D[(size_t)((i) + 1) * W + (size_t)((j) + 1)]
     for (int j = -1; j < tlen; ++j) AT(-1, j) = j + 1;
     for (int i = 0; i < qlen; ++i) {
@@ -52,6 +51,18 @@ int sdo_nw_path_counts(const char *q, int qlen, const char *t, int tlen, int *ma
             AT(i, j) = d;
         }
     }
+    return D;
+}
+
+/* Returns the edit distance; *matches = number of '=' columns, *columns = alignment length.
+ * Either sequence empty: main.py:30-33 returns (-1, "") -> identity 0; reported here as -1. */
+int sdo_nw_path_counts(const char *q, int qlen, const char *t, int tlen, int *matches, int *columns)
+{
+    *matches = 0; *columns = 0;
+    if (qlen <= 0 || tlen <= 0) return -1;
+    size_t W = (size_t)tlen + 1;
+    int *D = nw_matrix(q, qlen, t, tlen);
+    if (!D) return -2;
     int i = qlen - 1, j = tlen - 1, m = 0, c = 0;
     while (i >= 0 || j >= 0) {
         int cur = AT(i, j);
@@ -61,8 +72,57 @@ int sdo_nw_path_counts(const char *q, int qlen, const char *t, int tlen, int *ma
         ++c;
     }
     int dist = AT(qlen - 1, tlen - 1);
-#undef AT
     free(D);
     *matches = m; *columns = c;
     return dist;
+}
+
+/* The triple of every prefix pair (q[:i+1], t[:j+1]) at once, into qlen x tlen row-major arrays.  With edlib's
+ * boundary the matrix of a prefix pair is the top-left block of the full one, and the walk above is memoryless, so
+ * the triple of (i, j) is that of the walk started at (i, j): one step of the walk (the same tests in the same order)
+ * from the already-known triple of the cell it moves to.  A boundary cell (i, -1) or (-1, j) walks straight to the
+ * corner: no '=' column, i + 1 or j + 1 columns.  Returns 0, -1 when either sequence is empty, -2 without memory. */
+int sdo_nw_prefix_counts(const char *q, int qlen, const char *t, int tlen, int32_t *dist, int32_t *matches, int32_t *columns)
+{
+    if (qlen <= 0 || tlen <= 0) return -1;
+    size_t W = (size_t)tlen + 1, T = (size_t)tlen;
+    int *D = nw_matrix(q, qlen, t, tlen);
+    if (!D) return -2;
+#define CELL(i, j) ((size_t)(i) * T + (size_t)(j))
+    for (int i = 0; i < qlen; ++i)
+        for (int j = 0; j < tlen; ++j) {
+            int cur = AT(i, j), pi, pj, eq = 0;
+            if (AT(i - 1, j) + 1 == cur) { pi = i - 1; pj = j; }
+            else if (AT(i, j - 1) + 1 == cur) { pi = i; pj = j - 1; }
+            else { eq = AT(i - 1, j - 1) == cur; pi = i - 1; pj = j - 1; }
+            int pm = 0, pc = pi + pj + 2;                               /* boundary: i + 1 or j + 1 columns */
+            if (pi >= 0 && pj >= 0) { pm = matches[CELL(pi, pj)]; pc = columns[CELL(pi, pj)]; }
+            dist[CELL(i, j)] = cur; matches[CELL(i, j)] = pm + eq; columns[CELL(i, j)] = pc + 1;
+        }
+#undef CELL
+#undef AT
+    free(D);
+    return 0;
+}
+
+/* sdo_nw_path_counts over a pair list of packed sequences (offsets as sd_identity takes them), in parallel.
+ * Returns 0, or -2 when a pair's matrix could not be allocated. */
+int sdo_nw_path_counts_batch(const char *qtext, const int64_t *qoff, const char *ttext, const int64_t *toff,
+                             const int32_t *pair_q, const int32_t *pair_t, int64_t npairs,
+                             int32_t *dist, int32_t *matches, int32_t *columns)
+{
+    int status = 0;
+#pragma omp parallel for schedule(dynamic, 64)
+    for (int64_t p = 0; p < npairs; ++p) {
+        const int64_t qi = pair_q[p], ti = pair_t[p];
+        int m, c;
+        int d = sdo_nw_path_counts(qtext + qoff[qi], (int)(qoff[qi + 1] - qoff[qi]), ttext + toff[ti],
+                                   (int)(toff[ti + 1] - toff[ti]), &m, &c);
+        if (d == -2) {
+#pragma omp atomic write
+            status = -2;
+        }
+        dist[p] = d; matches[p] = m; columns[p] = c;
+    }
+    return status;
 }

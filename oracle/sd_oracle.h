@@ -27,6 +27,10 @@ int sdo_cli_main(int argc, char **argv);
 /* identity rescoring (sd_identity_oracle.c; main.py:29-60) */
 int sdo_nw_path_counts(const char *q, int qlen, const char *t, int tlen, int *matches, int *columns);
 int sdo_nw_uses_traceback(int qlen, int tlen);
+int sdo_nw_prefix_counts(const char *q, int qlen, const char *t, int tlen, int32_t *dist, int32_t *matches, int32_t *columns);
+int sdo_nw_path_counts_batch(const char *qtext, const int64_t *qoff, const char *ttext, const int64_t *toff,
+                             const int32_t *pair_q, const int32_t *pair_t, int64_t npairs,
+                             int32_t *dist, int32_t *matches, int32_t *columns);
 
 #ifdef __cplusplus
 }

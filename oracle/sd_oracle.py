@@ -40,6 +40,11 @@ def lib():
         _lib.sdo_postprocess.restype = C.c_int
         _lib.sdo_filter_rows.argtypes = [C.c_char_p, C.c_int, C.c_char_p, C.POINTER(C.c_int), C.c_int, C.c_int, C.POINTER(C.c_int)]
         _lib.sdo_filter_rows.restype = C.c_int
+        _lib.sdo_nw_prefix_counts.argtypes = [C.c_char_p, C.c_int, C.c_char_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
+        _lib.sdo_nw_prefix_counts.restype = C.c_int
+        _lib.sdo_nw_path_counts_batch.argtypes = [C.c_char_p, C.c_void_p, C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                  C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]
+        _lib.sdo_nw_path_counts_batch.restype = C.c_int
     return _lib
 
 
@@ -157,7 +162,7 @@ _ref_edlib = None
 
 
 def _counts(fn, q, t):
-    qb, tb = q.encode(), t.encode()
+    qb, tb = (s.encode() if isinstance(s, str) else bytes(s) for s in (q, t))
     m, c = C.c_int(), C.c_int()
     d = fn(qb, len(qb), tb, len(tb), C.byref(m), C.byref(c))
     return d, m.value, c.value
@@ -168,6 +173,35 @@ def nw_path_counts(q, t):
     f = lib().sdo_nw_path_counts
     f.argtypes = [C.c_char_p, C.c_int, C.c_char_p, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]
     return _counts(f, q, t)
+
+
+def nw_prefix_counts(q, t):
+    """The triple of nw_path_counts for every prefix pair (q[:i+1], t[:j+1]) -> (distance, matches, columns), three int32
+    numpy arrays of shape [len(q), len(t)]; q and t non-empty str or bytes."""
+    import numpy as np
+    qb = q.encode() if isinstance(q, str) else bytes(q)
+    tb = t.encode() if isinstance(t, str) else bytes(t)
+    out = [np.zeros((len(qb), len(tb)), np.int32) for _ in range(3)]
+    st = lib().sdo_nw_prefix_counts(qb, len(qb), tb, len(tb), *[C.c_void_p(a.ctypes.data) for a in out])
+    if st:
+        raise RuntimeError("sdo_nw_prefix_counts failed (%d)" % st)
+    return tuple(out)
+
+
+def nw_path_counts_batch(qtext, qoff, ttext, toff, pair_q, pair_t):
+    """nw_path_counts of every pair (qtext[qoff[pair_q[k]]:qoff[pair_q[k]+1]], the same for t), packed inputs as
+    sd_identity takes them, computed in parallel -> (distance, matches, columns) int32 arrays."""
+    import numpy as np
+    qo, to = np.ascontiguousarray(qoff, np.int64), np.ascontiguousarray(toff, np.int64)
+    pq, pt = np.ascontiguousarray(pair_q, np.int32), np.ascontiguousarray(pair_t, np.int32)
+    assert pq.shape == pt.shape and (pq.size == 0 or (0 <= pq.min() and pq.max() < len(qo) - 1 and 0 <= pt.min() and pt.max() < len(to) - 1))
+    out = [np.zeros(len(pq), np.int32) for _ in range(3)]
+    st = lib().sdo_nw_path_counts_batch(bytes(qtext), C.c_void_p(qo.ctypes.data), bytes(ttext), C.c_void_p(to.ctypes.data),
+                                        C.c_void_p(pq.ctypes.data), C.c_void_p(pt.ctypes.data), C.c_int64(len(pq)),
+                                        *[C.c_void_p(a.ctypes.data) for a in out])
+    if st:
+        raise RuntimeError("sdo_nw_path_counts_batch failed (%d)" % st)
+    return tuple(out)
 
 
 def nw_uses_traceback(qlen, tlen):

@@ -13,6 +13,8 @@
 // smallest distance and, among equal distances, edlib's preferred move, and drags that move's M along.
 #pragma once
 #include <cstdint>
+#include <cstdio>
+#include <cstdlib>
 #if defined(__CUDACC__)
 #define SDI_HD __host__ __device__ __forceinline__
 #else
@@ -98,6 +100,20 @@ inline int nw_choose_rows(const int64_t *qoff, int64_t nq)
         if (cost < best) { best = cost; best_r = cand; }
     }
     return best_r;
+}
+
+// The geometries compiled into the library, as (lanes per pair L, rows per lane R).
+constexpr int NW_GEOMS[5][2] = {{8, 8}, {8, 16}, {8, 24}, {16, 12}, {32, 6}};
+
+// (L, R) of a batch, for the launcher and the emulator alike: NW_LANES lanes with the strip nw_choose_rows picks,
+// unless SD_NW_GEOM=L,R asks for another geometry (tests and experiments).  Returns false, with L and R as asked,
+// when that geometry is not compiled.
+inline bool nw_choose_geometry(const int64_t *qoff, int64_t nq, int &L, int &R)
+{
+    L = NW_LANES; R = nw_choose_rows(qoff, nq);
+    if (const char *e = getenv("SD_NW_GEOM")) { int l = 0, r = 0; if (sscanf(e, "%d,%d", &l, &r) == 2) { L = l; R = r; } }
+    for (const auto &g : NW_GEOMS) if (g[0] == L && g[1] == R) return true;
+    return false;
 }
 
 // Above 1 MiB of traceback state edlib switches to Hirschberg splitting (edlib.cpp:1187-1191), whose path may differ.

@@ -30,7 +30,7 @@ __global__ void __launch_bounds__(256) identity_kernel(IdentityArgs a)
 {
     constexpr int G = 32 / L;
     const int lane = threadIdx.x & 31, gl = lane % L, sub = lane / L;
-    const unsigned mask = ((1u << L) - 1u) << (sub * L);
+    const unsigned mask = (0xffffffffu >> (32 - L)) << (sub * L);     // this group's lanes; no shift by 32 when L = 32
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int64_t group = warp * G + sub, ngroups = (((int64_t)gridDim.x * blockDim.x) >> 5) * G;
     uint32_t *scratch = a.scratch ? a.scratch + group * a.scratch_stride : nullptr;
@@ -115,15 +115,13 @@ int cuda_identity(const IdentityArgs &h, int max_qlen, int max_tlen, int device,
         const auto t_begin = std::chrono::steady_clock::now();
         auto since = [&] { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count(); };
         const size_t qbytes = (size_t)h.qoff[h.nq], tbytes = (size_t)h.toff[h.nt];
-        int R = nw_choose_rows(h.qoff, h.nq), L = NW_LANES;
-        if (const char *e = getenv("SD_NW_GEOM")) { int l = 0, r = 0; if (sscanf(e, "%d,%d", &l, &r) == 2) { L = l; R = r; } }   // experiments
-        void (*kernel)(IdentityArgs) = nullptr;
+        int L = 0, R = 0;
+        if (!nw_choose_geometry(h.qoff, h.nq, L, R)) { err = "unsupported SD_NW_GEOM"; return 4; }
+        void (*kernel)(IdentityArgs) = identity_kernel<6, 32>;      // one per NW_GEOMS entry
         if (L == 8 && R == 8) kernel = identity_kernel<8, 8>;
         else if (L == 8 && R == 16) kernel = identity_kernel<16, 8>;
         else if (L == 8 && R == 24) kernel = identity_kernel<24, 8>;
         else if (L == 16 && R == 12) kernel = identity_kernel<12, 16>;
-        else if (L == 32 && R == 6) kernel = identity_kernel<6, 32>;
-        else { err = "unsupported SD_NW_GEOM"; return 4; }
         const int threads = 256, wpb = threads / 32 * (32 / L);                                    // pairs in flight per block
         int resident = 1;                                           // grid-stride kernel: exactly one resident wave of blocks
         SDI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kernel, threads, 0));
@@ -164,8 +162,8 @@ int cuda_identity(const IdentityArgs &h, int max_qlen, int max_tlen, int device,
         SDI_CUDA(cudaStreamSynchronize(nullptr));
         float ms = 0; SDI_CUDA(cudaEventElapsedTime(&ms, ar.e0, ar.e1));
         if (kernel_ms) *kernel_ms = ms;
-        if (prof) fprintf(stderr, "[sd_b200 profile] sd_identity: pairs %ld R %d blocks %ld  h2d issue %.2f ms, kernel %.3f ms, total %.2f ms\n",
-                          (long)h.npairs, R, (long)blocks, t_h2d, ms, since());
+        if (prof) fprintf(stderr, "[sd_b200 profile] sd_identity: pairs %ld L %d R %d blocks %ld x %d pairs  h2d issue %.2f ms, kernel %.3f ms, total %.2f ms\n",
+                          (long)h.npairs, L, R, (long)blocks, wpb, t_h2d, ms, since());
     } catch (PlanError &e) { err = e.msg; return 4; }
     return 0;
 }

@@ -429,13 +429,12 @@ private:
 
 Backend *make_emu_backend() { return new EmuBackend(); }
 
-// Host emulation of identity_kernel (identity_kernels.cu): the same strips, tiles, wavefront steps and spill row,
-// with the NW_LANES lanes of a group walked in descending order so that lane l reads lane l-1's bottom cell of the
+// Host emulation of identity_kernel<R, L> (identity_kernels.cu): the same strips, tiles, wavefront steps and spill
+// row, with the L lanes of a group walked in descending order so that lane l reads lane l-1's bottom cell of the
 // previous step, exactly what the SHFL.UP delivers on the device.
-template <int R>
+template <int R, int L>
 static void emu_identity_pair(const char *q, int qlen, const char *t, int tlen, std::vector<uint32_t> &scratch, int &m, int &d)
 {
-    constexpr int L = NW_LANES;
     const int ntiles = (qlen + L * R - 1) / (L * R);
     NwLane<R> st[L];
     uint32_t bottom[L];
@@ -459,23 +458,24 @@ static void emu_identity_pair(const char *q, int qlen, const char *t, int tlen, 
     d = (int)(v >> NW_DSHIFT); m = (int)(v & 0xffffu);
 }
 
-int emu_identity(const IdentityArgs &a, int max_qlen, int max_tlen, double *kernel_ms, std::string &)
+int emu_identity(const IdentityArgs &a, int max_qlen, int max_tlen, double *kernel_ms, std::string &err)
 {
     (void)max_qlen;
-    const int R = nw_choose_rows(a.qoff, a.nq);
+    int L = 0, R = 0;
+    if (!nw_choose_geometry(a.qoff, a.nq, L, R)) { err = "unsupported SD_NW_GEOM"; return 4; }
+    if (getenv("SD_PROFILE")) fprintf(stderr, "[sd_b200 profile] sd_identity (emulator): pairs %ld L %d R %d\n", (long)a.npairs, L, R);
+    auto pair = emu_identity_pair<6, 32>;                   // one per NW_GEOMS entry
+    if (L == 8 && R == 8) pair = emu_identity_pair<8, 8>;
+    else if (L == 8 && R == 16) pair = emu_identity_pair<16, 8>;
+    else if (L == 8 && R == 24) pair = emu_identity_pair<24, 8>;
+    else if (L == 16 && R == 12) pair = emu_identity_pair<12, 16>;
     std::vector<uint32_t> scratch((size_t)max_tlen + 32);
     for (int64_t p = 0; p < a.npairs; ++p) {
         const int64_t qi = a.pair_q ? a.pair_q[p] : p / a.nt, ti = a.pair_q ? a.pair_t[p] : p % a.nt;
         const char *q = a.qtext + a.qoff[qi], *t = a.ttext + a.toff[ti];
         const int qlen = (int)(a.qoff[qi + 1] - a.qoff[qi]), tlen = (int)(a.toff[ti + 1] - a.toff[ti]);
         int m = 0, d = -1;
-        if (qlen > 0 && tlen > 0) {
-            switch (R) {
-            case 8: emu_identity_pair<8>(q, qlen, t, tlen, scratch, m, d); break;
-            case 16: emu_identity_pair<16>(q, qlen, t, tlen, scratch, m, d); break;
-            default: emu_identity_pair<24>(q, qlen, t, tlen, scratch, m, d); break;
-            }
-        }
+        if (qlen > 0 && tlen > 0) pair(q, qlen, t, tlen, scratch, m, d);
         a.matches[p] = m; a.columns[p] = d < 0 ? 0 : m + d;
         if (a.distance) a.distance[p] = d;
     }

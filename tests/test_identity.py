@@ -367,7 +367,8 @@ def test_gpu_command_line_end_to_end_equals_reference_golden_file(tmp_path):
 
 @pytest.mark.gpu
 def test_gpu_identity_full_size_properties():
-    """Config-2-sized rescoring (12k intervals x 24 monomers, plain): properties that need no oracle."""
+    """Config-2-sized rescoring (12k intervals x 24 monomers, plain): properties that need no oracle, and every pair
+    against the oracle."""
     from stringdecomposer_b200 import synth
     r = random.Random(2)
     _, mons = sd.read_fasta(os.path.join(G, "DXZ1_star_monomers.fa"))
@@ -382,10 +383,13 @@ def test_gpu_identity_full_size_properties():
     assert (np.argmax(m / c, axis=1) == np.array(truth)).mean() > 0.99
     again = sd.nw_identity(qs[:500], rows)
     assert (again["matches"] == res["matches"][:500 * len(rows)]).all()
-    samp = r.sample(range(len(qs)), 40)
-    for i in samp:
-        for j in (truth[i], (truth[i] + 5) % len(rows)):
-            assert (d[i, j], m[i, j], c[i, j]) == O.nw_path_counts(qs[i], rows[j])
+    qb, qo = cv._pack(qs)
+    tb, to = cv._pack(rows)
+    want = O.nw_path_counts_batch(qb, qo, tb, to, np.repeat(np.arange(len(qs)), len(rows)), np.tile(np.arange(len(rows)), len(qs)))
+    for name, got, w in zip(("distance", "matches", "columns"), (res["distance"], res["matches"], res["columns"]), want):
+        bad = np.flatnonzero(got != w)
+        assert len(bad) == 0, "%s: %d pairs differ from the oracle, first (interval %d, row %d): %d != %d" % (
+            name, len(bad), bad[0] // len(rows), bad[0] % len(rows), got[bad[0]], w[bad[0]])
 
 
 def test_raw_file_is_streamed_in_chunks_of_whole_reads(tmp_path):
